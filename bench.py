@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- SEA hot-path throughput on B200 (BASELINE.json metric: decode & encode Msamples/s, fraction of roofline).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W]            our arm (one process per GPU under torchrun for N > 1)
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--dump-outputs DIR]   our arm (one process per GPU under torchrun for N > 1)
   python bench.py --impl reference [--gpus N --steps K --warmup W] the reference's own CPU decoder on the host cores
 
 A "step" is one pass of the hot path over one batch of synthetic streams.  Headline (`value`) = batch decode of BASELINE
@@ -37,11 +37,13 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the benchmark leaves the tree as it found it (no __pycache__ of the modules it imports)
 
 RATE, CHANNELS, SECONDS = 44100, 2, 60
 ALG_OPS_PER_CAND_SAMPLE = 49  # SURVEY.md 8d op count of encoder_base.rs:64-89 + lms.rs
 CBR_ROWS = [1, 2, 3, 4, 5, 6, 7, 8]
 VBR_ROWS = [1.5, 2.0, 2.5, 3.0, 3.5, 4.0, 5.0, 6.0, 7.0, 7.3]
+DUMP_STREAMS, DUMP_WINDOW = 4096, 2048  # --dump-outputs: at most 4096 x 2048 samples, 32 MB as float32
 
 
 def measured_peaks():
@@ -272,10 +274,35 @@ def decode_device(ctx, sea, stride, lens, headers, pcm_out, spp, n):
     return got, ctx.last_kernel_ms
 
 
+def dump_outputs(out_dir, torch, pcm_out, got, n, spp):
+    """Writes what the timed decode returned in its last step, as float32 / float64 .npy files: the samples decoded per stream
+    and, for every stream (a seeded choice of DUMP_STREAMS when there are more), one seeded window of its decoded PCM.  The
+    windows depend only on the stream count and length, so two builds run with the same arguments compare file for file."""
+    os.makedirs(out_dir, exist_ok=True)
+    rng = np.random.default_rng(0)
+    streams = np.arange(n, dtype=np.int64) if n <= DUMP_STREAMS else np.sort(rng.choice(n, DUMP_STREAMS, replace=False))
+    width = min(spp, DUMP_WINDOW)
+    starts = rng.integers(0, spp - width + 1, size=streams.size, dtype=np.int64)
+    idx = streams[:, None] * spp + starts[:, None] + np.arange(width, dtype=np.int64)
+    windows = pcm_out[torch.from_numpy(idx).to(pcm_out.device)].float().cpu().numpy()
+    np.save(os.path.join(out_dir, "samples_per_stream.npy"), np.asarray(got, dtype=np.float64))
+    np.save(os.path.join(out_dir, "pcm_windows.npy"), windows)
+    np.save(os.path.join(out_dir, "pcm_window_stream_and_start.npy"), np.stack([streams, starts], axis=1).astype(np.float64))
+
+
+def positive_int(text):
+    v = int(text)
+    if v < 1:
+        raise argparse.ArgumentTypeError("must be at least 1")
+    return v
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=40)  # ~0.6 s timed region: enough nvidia-smi clock samples
+    ap.add_argument("--steps", type=positive_int, default=40,  # ~0.6 s timed region: enough nvidia-smi clock samples
+                    help="timed steps of the headline decode (value, ms_per_step); the secondary sections time their own "
+                         "bounded repeat counts (1 to 10)")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--streams", type=int, default=4096, help="decode streams per GPU (config 4, weak) and in total (strong)")
@@ -286,6 +313,8 @@ def main():
     ap.add_argument("--skip-sweep", action="store_true")
     ap.add_argument("--skip-cpu", action="store_true")
     ap.add_argument("--skip-e2e", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write a seeded sample of what the last timed decode step returned "
+                                                          "(rank 0) to DIR/*.npy")
     args = ap.parse_args()
 
     from sea_codec_b200 import dist
@@ -377,6 +406,8 @@ def main():
     ms_per_step = ms_total / args.steps
     value = W * samples_per_step / (ms_per_step * 1e-3) / 1e6
     assert np.all(got == spp)
+    if args.dump_outputs and info.rank == 0:
+        dump_outputs(args.dump_outputs, torch, pcm_out, got, n, spp)
     k_ms = float(np.mean(kernel_ms))
     achieved = alg_bytes / (k_ms * 1e-3) / 1e9
     roofline = {"bound": "hbm", "kernel": "decode_unrolled_kernel<2,3,pair-repl,S=4> (+ decode_staged_kernel<2,0> for the partial last chunks, "

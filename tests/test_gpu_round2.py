@@ -11,7 +11,7 @@ import pytest
 
 import sea_codec_b200 as S
 from sea_codec_b200 import api, synth
-from util import gen_test_signal
+from util import gen_test_signal, reference_c_result, sha
 
 pytestmark = pytest.mark.gpu
 
@@ -29,22 +29,23 @@ def test_gpu_encoder_lms_against_the_reference_decoder(ctx, oracle, channels, bi
     state the REFERENCE decoder holds at each chunk end (captured before its free, c/sea.h:147-185) equals, mod 2^16
     (lms.rs:64-78), the LMS block the GPU encoder wrote into the next chunk header (file.rs:146-149).  That checks the encoder's
     dequantise / predict / clamp / update path (encoder_base.rs:73-88, lms.rs:33-51) against reference code with no restatement
-    in between; the history half is also visible black-box in the PCM c/sea.h emits."""
-    if not oracle.have_ref():
-        pytest.skip("oracle/_ref not built")
+    in between; the history half is also visible black-box in the PCM c/sea.h emits.  Without oracle/_ref the state and PCM
+    come from the record (util.reference_c_result); recorded from the oracle, they pin the GPU encoder and decoder to the
+    oracle's bytes and decode."""
     n_chunks, frames = 5, 5120 * 4 + 1000  # whole scale-factor blocks only (c/sea.h:168)
     pcm = synth.gen_stream(900 + channels * 10 + bits, frames, channels, 44100)
     enc = ctx.sea_encode(pcm, 44100, channels, S.EncoderSettings(residual_bits=float(bits)))
-    info, lms = oracle.ref_c_decode_lms(enc)
+    pcm_sha, lms = reference_c_result(oracle, f"gpu_encoder_lms/ch{channels}_b{bits}", enc, lms=True)
     hdr = oracle.chunk_header_lms(enc)
-    assert lms.shape == hdr.shape == (n_chunks, channels, 8)
-    assert np.array_equal(lms[:-1].astype(np.int16), hdr[1:]), "encoder's chunk-header LMS != the reference decoder's end-of-chunk state"
-    out = info.samples.reshape(-1, channels)
+    assert hdr.shape == (n_chunks, channels, 8) and lms.shape == (n_chunks - 1, channels, 8)
+    assert np.array_equal(lms, hdr[1:]), "encoder's chunk-header LMS != the reference decoder's end-of-chunk state"
+    # the GPU decoder agrees with the reference decoder on the GPU encoder's bytes, so its PCM stands for c/sea.h's below
+    dec = ctx.sea_decode(enc).samples
+    assert sha(dec) == pcm_sha
+    out = dec.reshape(-1, channels)
     for k in range(1, n_chunks):
         assert np.array_equal(hdr[k][:, :4].T, out[k * 5120 - 4: k * 5120])
     assert np.array_equal(hdr[0][:, 4:], np.tile(np.array([0, 0, -8192, 16384], dtype=np.int16), (channels, 1)))
-    # and the GPU decoder agrees with the reference decoder on the GPU encoder's bytes
-    assert np.array_equal(ctx.sea_decode(enc).samples, info.samples)
 
 
 def test_vbr_bytes_equal_the_oracle_even_with_ties_and_ties_are_counted_per_stream(ctx, oracle):

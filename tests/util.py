@@ -1,15 +1,37 @@
 """Shared helpers of the test-suite."""
 import hashlib
+import json
 import os
 import subprocess
 
 import numpy as np
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+REFERENCE_C_GOLDEN = os.path.join(ROOT, "tests", "golden", "reference_c.json")
 
 
 def sha(b) -> str:
     return hashlib.sha256(np.ascontiguousarray(b).tobytes() if isinstance(b, np.ndarray) else b).hexdigest()
+
+
+def reference_c_result(oracle, key: str, encoded: bytes, lms: bool = False):
+    """What the reference's own C decoder (c/sea.h) makes of `encoded`: (sha256 of its PCM, and with lms=True the LMS state it
+    holds at the end of every chunk but the last, int16 [chunk][channel][8] -- history[4] then weights[4], mod 2^16).
+    Where oracle/_ref is built, c/sea.h runs and must agree with tests/golden/reference_c.json; elsewhere the recorded result
+    is used.  Either way `encoded` must be the very input the record belongs to.  The record's "source" says where it came
+    from: while it is the oracle rather than c/sea.h, a test without oracle/_ref compares with the oracle's recorded result."""
+    with open(REFERENCE_C_GOLDEN) as f:
+        rec = json.load(f)["cases"][key]
+    assert sha(encoded) == rec["sea_sha"], f"{key}: not the input whose c/sea.h result is recorded"
+    want_lms = np.array(rec["lms"], dtype=np.int16) if lms else None
+    if oracle.have_ref():
+        if lms:
+            info, states = oracle.ref_c_decode_lms(encoded)
+            assert np.array_equal(states[:-1].astype(np.int16), want_lms), f"{key}: c/sea.h LMS differs from the record"
+        else:
+            info = oracle.ref_c_decode(encoded)
+        assert sha(info.samples) == rec["pcm_sha"], f"{key}: c/sea.h PCM differs from the record"
+    return (rec["pcm_sha"], want_lms) if lms else rec["pcm_sha"]
 
 
 def gen_test_signal(channels: int, frames: int, rate: int = 44100, seed: int = 1) -> np.ndarray:
