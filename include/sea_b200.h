@@ -213,6 +213,23 @@ int sea_b200_decode_range(sea_b200_ctx *ctx, const uint8_t *sea, uint64_t len, u
                           uint32_t flags, int16_t *pcm, uint64_t pcm_cap_samples, uint64_t *n_samples, uint32_t *sample_rate,
                           uint32_t *channels);
 
+/* Output format bit of `flags` (combinable with SEA_B200_RANGE_SKIP_METADATA, which means what it means for decode_range). */
+#define SEA_B200_WINDOW_F32_PLANAR 2u
+/* n_windows frame windows of device-resident streams in one call (e.g. fixed-length training crops of a corpus kept in HBM).
+ * Streams are described as for sea_b200_decode_batch_device (d_sea + host offsets / lengths, n_streams * 22 header bytes on
+ * the host).  Window w = frames [first_frames[w], first_frames[w] + n_frames[w]) of stream window_stream[w]; several windows
+ * may name the same stream.  Output slot w starts at element out_offsets[w] of d_out (device memory):
+ *   default:                    int16, interleaved  [n_frames[w]][channels]   (the library's PCM layout)
+ *   SEA_B200_WINDOW_F32_PLANAR: float32, planar     [channels][n_frames[w]], value = sample / 32768.0f
+ * The first frames_out[w] frames of a slot are what sea_b200_decode_range(stream, first, n, flags & SKIP_METADATA) returns;
+ * frames the stream does not have (past its end, clamped as decode_range clamps them) are written as zeros.  Bytes of d_out
+ * outside the slots are never written.  Only the chunks that cover a window are decoded.  A window_stream index >= n_streams
+ * or an unknown flag bit is SEA_B200_ERR_INVALID_PARAMETERS; a bad chunk inside a window gives decode_range's code for it. */
+int sea_b200_decode_windows_device(sea_b200_ctx *ctx, uint32_t n_streams, const uint8_t *d_sea, const uint64_t *sea_offsets,
+                                   const uint64_t *sea_lens, const uint8_t *headers, uint32_t n_windows,
+                                   const uint32_t *window_stream, const uint64_t *first_frames, const uint32_t *n_frames,
+                                   uint32_t flags, void *d_out, const uint64_t *out_offsets, uint64_t *frames_out);
+
 /* ---------------------------------------------------------------- the reference's existing foreign surfaces */
 
 /* src/wasm_api.rs:32-111 (wasm_sea_encode / wasm_sea_decode / allocate / deallocate / setup) with the same argument lists,

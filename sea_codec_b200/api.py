@@ -26,6 +26,7 @@ OK = 0
 ERR_READ, ERR_INVALID_PARAMETERS, ERR_INVALID_FILE, ERR_INVALID_FRAME = -1, -2, -3, -4
 ERR_ENCODER_CLOSED, ERR_UNSUPPORTED_VERSION, ERR_TOO_MANY_FRAMES, ERR_METADATA_TOO_LARGE, ERR_IO = -5, -6, -7, -8, -9
 ERR_CAPACITY, ERR_DOMAIN, ERR_CUDA, ERR_NOMEM = -20, -21, -30, -31
+RANGE_SKIP_METADATA, WINDOW_F32_PLANAR = 1, 2  # flag bits of decode_range / decode_windows_device
 
 _NAMES = {
     ERR_READ: "ReadError", ERR_INVALID_PARAMETERS: "InvalidParameters", ERR_INVALID_FILE: "InvalidFile",
@@ -135,6 +136,8 @@ SYMBOLS = {
     "sea_b200_decoder_decode_chunks": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_int64, C.c_void_p, C.c_uint64, _u64p]),
     "sea_b200_decode_range": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint64, C.c_uint64, C.c_uint32, C.c_void_p, C.c_uint64,
                                         _u64p, _u32p, _u32p]),
+    "sea_b200_decode_windows_device": (C.c_int, [C.c_void_p, C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32,
+                                                 C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p]),
     "sea_b200_wasm_setup": (None, []),
     "sea_b200_wasm_sea_encode": (C.c_size_t, [C.c_void_p, C.c_size_t, C.c_uint32, C.c_uint32, C.c_float, C.c_bool, C.c_void_p, C.c_size_t]),
     "sea_b200_wasm_sea_decode": (C.c_size_t, [C.c_void_p, C.c_size_t, C.c_void_p, C.c_size_t, _u32p, _u32p]),
@@ -397,6 +400,28 @@ class Context:
                                                          hd.ctypes.data, C.c_void_p(d_pcm), po.ctypes.data,
                                                          caps.ctypes.data if caps is not None else None, n.ctypes.data))
         return n
+
+    def decode_windows_device(self, d_sea: int, sea_offsets, sea_lens, headers: np.ndarray, window_stream, first_frames, n_frames,
+                              d_out: int, out_offsets, float32_planar: bool = False, skip_metadata: bool = False) -> np.ndarray:
+        """Frame windows [first_frames[w], first_frames[w] + n_frames[w]) of device-resident streams window_stream[w] (described as
+        for decode_batch_device) into slots of d_out starting at element out_offsets[w]: int16 [n_frames][channels], or with
+        float32_planar float32 [channels][n_frames] = sample / 32768.  Each slot holds what decode_range returns for its window,
+        then zeros.  Returns frames_out, the real frames per window."""
+        so, sl = _u64(sea_offsets), _u64(sea_lens)
+        hd = np.ascontiguousarray(headers, dtype=np.uint8)
+        ws = np.ascontiguousarray(window_stream, dtype=np.uint32)
+        ff, oo = _u64(first_frames), _u64(out_offsets)
+        nf = np.ascontiguousarray(n_frames, dtype=np.uint32)
+        if not (ws.size == ff.size == nf.size == oo.size):
+            raise SeaError(ERR_INVALID_PARAMETERS, "window arrays differ in length")
+        if so.size != sl.size or hd.size < so.size * 22:
+            raise SeaError(ERR_INVALID_PARAMETERS, "stream arrays differ in length")
+        flags = (WINDOW_F32_PLANAR if float32_planar else 0) | (RANGE_SKIP_METADATA if skip_metadata else 0)
+        out = np.zeros(ws.size, dtype=np.uint64)
+        self._check(self._L.sea_b200_decode_windows_device(self._h, so.size, C.c_void_p(d_sea), so.ctypes.data, sl.ctypes.data,
+                                                           hd.ctypes.data, ws.size, ws.ctypes.data, ff.ctypes.data, nf.ctypes.data, flags,
+                                                           C.c_void_p(d_out), oo.ctypes.data, out.ctypes.data))
+        return out
 
 
 class MultiContext:

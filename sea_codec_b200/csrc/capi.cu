@@ -77,6 +77,7 @@ struct sea_b200_ctx {
     size_t h_errs_cap = 0;
     std::vector<cudaEvent_t> grp_ev;
     cudaStream_t up = nullptr;  // uploads of a pipelined batch run ahead of the lanes on their own stream
+    DevBuf win, win_desc;       // sea_b200_decode_windows_device: decoded covering chunks of a group of windows, their descriptors
     std::string last_error;
     uint64_t launches = 0;
     double last_kernel_ms = 0.0;
@@ -791,6 +792,8 @@ void sea_b200_ctx_destroy(sea_b200_ctx *ctx)
         ctx->pipe.out[i].release();
     }
     ctx->pipe.state.release();
+    ctx->win.release();
+    ctx->win_desc.release();
     if (ctx->aux.stream) { cudaStreamSynchronize(ctx->aux.stream); cudaStreamDestroy(ctx->aux.stream); }
     if (ctx->aux.side) { cudaStreamSynchronize(ctx->aux.side); cudaStreamDestroy(ctx->aux.side); }
     if (ctx->aux.ev_fork) cudaEventDestroy(ctx->aux.ev_fork);
@@ -1197,6 +1200,140 @@ int sea_b200_decode(sea_b200_ctx *ctx, const uint8_t *sea, uint64_t len, int16_t
         return SEA_B200_OK;
     }
     return sea_b200_decode_batch(ctx, 1, sea, &off, &len, pcm, &poff, &pcm_cap_samples, n_samples);
+}
+
+// ------------------------------------------------------------------------------------------------ frame windows
+
+// Every non-empty window becomes one DecStream over the chunks that cover it (plan_range, the arithmetic of decode_range), decoded
+// by run_decode into a scratch buffer exactly as decode_range decodes its sub-file; window_extract_kernel then cuts each slot out.
+// Windows go in index order in groups whose covering ranges fit the scratch cap (one run_decode + one cut per group).
+int sea_b200_decode_windows_device(sea_b200_ctx *ctx, uint32_t n_streams, const uint8_t *d_sea, const uint64_t *sea_offsets,
+                                   const uint64_t *sea_lens, const uint8_t *headers, uint32_t n_windows, const uint32_t *window_stream,
+                                   const uint64_t *first_frames, const uint32_t *n_frames, uint32_t flags, void *d_out,
+                                   const uint64_t *out_offsets, uint64_t *frames_out)
+{
+    if (!ctx || !sea_offsets || !sea_lens || !headers) return SEA_B200_ERR_INVALID_PARAMETERS;
+    if (flags & ~(SEA_B200_RANGE_SKIP_METADATA | SEA_B200_WINDOW_F32_PLANAR))
+        return fail(ctx, SEA_B200_ERR_INVALID_PARAMETERS, "unknown flag bits");
+    if (n_windows == 0) return SEA_B200_OK;
+    if (!window_stream || !first_frames || !n_frames || !d_out || !out_offsets) return SEA_B200_ERR_INVALID_PARAMETERS;
+    if (frames_out) memset(frames_out, 0, sizeof(uint64_t) * n_windows);
+    const bool planar = flags & SEA_B200_WINDOW_F32_PLANAR;
+    if (reinterpret_cast<uintptr_t>(d_out) % (planar ? sizeof(float) : sizeof(int16_t)))
+        return fail(ctx, SEA_B200_ERR_INVALID_PARAMETERS, "d_out is not aligned to its element type");
+    for (uint32_t w = 0; w < n_windows; w++)
+        if (window_stream[w] >= n_streams)
+            return fail(ctx, SEA_B200_ERR_INVALID_PARAMETERS, "window " + std::to_string(w) + ": stream index out of range");
+    std::vector<sea_b200_header> hs(n_streams);
+    uint64_t sea_len = 0;
+    for (uint32_t i = 0; i < n_streams; i++) {  // as plan_decode checks them
+        const uint64_t len = sea_lens[i];
+        int rc = parse_file_header(headers + (size_t)i * kFileHeaderBytes, len < 22 ? len : 22, &hs[i]);
+        if (rc) return fail(ctx, rc, "stream " + std::to_string(i) + ": bad .sea header (file.rs:40-72)");
+        sea_len = std::max(sea_len, sea_offsets[i] + len);
+    }
+    std::vector<RangePlan> plans(n_windows);
+    for (uint32_t w = 0; w < n_windows; w++) {
+        const uint32_t s = window_stream[w];
+        int rc = plan_range(hs[s], sea_lens[s], first_frames[w], n_frames[w], flags & SEA_B200_RANGE_SKIP_METADATA, &plans[w]);
+        if (rc) return fail(ctx, rc, "window " + std::to_string(w) + ": metadata runs past the end of the stream");
+        if (plans[w].want && plans[w].sub_frames > 0xffffffffull)
+            return fail(ctx, SEA_B200_ERR_TOO_MANY_FRAMES, "window " + std::to_string(w) + ": covering chunks longer than 2^32 frames");
+    }
+    CU(cudaSetDevice(ctx->device));
+
+    // scratch samples per group: 2 GiB of int16 (SEA_B200_WIN_SCRATCH_SAMPLES: tests, tuning); a window larger than that is a group
+    uint64_t cap = 1ull << 30;
+    if (const char *env = getenv("SEA_B200_WIN_SCRATCH_SAMPLES")) cap = std::max<uint64_t>(1, strtoull(env, nullptr, 10));
+    auto region = [&](uint32_t w) -> uint64_t {  // rows of the lane-per-chunk kernels' 256-bit stores: 16-sample aligned
+        return plans[w].want ? (plans[w].sub_frames * hs[window_stream[w]].channels + 15u) & ~15ull : 0u;
+    };
+    const bool trace = getenv("SEA_B200_TRACE") != nullptr;
+    double decode_ms = 0.0, extract_ms = 0.0;
+    for (uint32_t w0 = 0, g = 0; w0 < n_windows; g++) {
+        uint32_t w1 = w0;
+        uint64_t scratch = 0;
+        while (w1 < n_windows && (w1 == w0 || scratch + region(w1) <= cap)) scratch += region(w1++);
+        DecodeJob job;
+        std::vector<WinDesc> desc;
+        uint64_t chains = 0, max_slot = 0, off = 0;
+        for (uint32_t w = w0; w < w1; w++) {
+            const RangePlan &r = plans[w];
+            const uint32_t s = window_stream[w];
+            const sea_b200_header &h = hs[s];
+            WinDesc wd = {};
+            wd.dst = out_offsets[w];
+            wd.frames = n_frames[w];
+            wd.channels = h.channels;
+            wd.real = (uint32_t)r.want;
+            if (r.want) {
+                DecStream d;
+                memset(&d, 0, sizeof(d));
+                d.data_off = sea_offsets[s] + r.b0;
+                d.data_len = r.b1 - r.b0;
+                d.pcm_off = off;
+                d.total_frames = (uint32_t)r.sub_frames;  // whole covering chunks: a chunk's layout depends on its own frame count
+                d.n_chunks = (uint32_t)(r.k1 - r.k0);
+                d.chain_begin = (uint32_t)chains;
+                d.chunk_size = h.chunk_size;
+                d.frames_per_chunk = h.frames_per_chunk;
+                d.channels = h.channels;
+                if (job.streams.empty()) job.first = h;
+                else if (h.channels != job.first.channels || h.chunk_size != job.first.chunk_size || h.frames_per_chunk != job.first.frames_per_chunk)
+                    job.uniform = false;
+                job.streams.push_back(d);
+                chains += (uint64_t)d.n_chunks * h.channels;
+                if (chains > 0xfffffff0ull) return fail(ctx, SEA_B200_ERR_INVALID_PARAMETERS, "window group too large (2^32 chains)");
+                wd.src = off + r.skip * h.channels;
+                off += region(w);
+            }
+            if (wd.frames) {
+                desc.push_back(wd);
+                max_slot = std::max(max_slot, (uint64_t)wd.frames * wd.channels);
+            }
+        }
+        job.total_chains = chains;
+        // the cut reads whole 16-byte vectors: up to 16 samples past a window's covering range
+        CU(ctx->win.reserve((off + 64) * sizeof(int16_t)));
+        float ms_dec = 0.f, ms_cut = 0.f;
+        if (!job.streams.empty()) {
+            const DecStream &d0 = job.streams[0];  // its first chunk's header word picks the specialised kernel
+            uint32_t hdr_word = 0;
+            bool have = false;
+            if (d0.data_len >= 4) {
+                uint8_t b[4];
+                CU(cudaMemcpyAsync(b, d_sea + d0.data_off, 4, cudaMemcpyDeviceToHost, ctx->stream));
+                CU(cudaStreamSynchronize(ctx->stream));
+                hdr_word = (uint32_t)b[0] | ((uint32_t)b[1] << 8) | ((uint32_t)b[2] << 16) | ((uint32_t)b[3] << 24);
+                have = true;
+            }
+            DecLane L = decode_lane(ctx, 0);
+            int rc = run_decode(ctx, L, job, d_sea, sea_len, ctx->win.as<int16_t>(), have, hdr_word);
+            if (rc) return rc;
+            ms_dec = (float)L.kernel_ms;
+        }
+        if (!desc.empty()) {
+            CU(ctx->win_desc.reserve(sizeof(WinDesc) * desc.size()));
+            CU(cudaMemcpyAsync(ctx->win_desc.p, desc.data(), sizeof(WinDesc) * desc.size(), cudaMemcpyHostToDevice, ctx->stream));
+            CU(cudaEventRecord(ctx->ev0, ctx->stream));
+            CU(launch_window_extract(ctx->win.as<int16_t>(), d_out, ctx->win_desc.as<WinDesc>(), (uint32_t)desc.size(), max_slot, planar,
+                                     ctx->stream));
+            ctx->launches++;
+            CU(cudaEventRecord(ctx->ev1, ctx->stream));
+            CU(cudaStreamSynchronize(ctx->stream));  // the next group reuses the scratch and the events
+            cudaEventElapsedTime(&ms_cut, ctx->ev0, ctx->ev1);
+        }
+        decode_ms += ms_dec;
+        extract_ms += ms_cut;
+        if (trace)
+            fprintf(stderr, "sea_b200 trace: window group %u: windows %u..%u, covering %llu samples, decode %.3f ms, extract %.3f ms\n", g, w0,
+                    w1 - 1, (unsigned long long)off, ms_dec, ms_cut);
+        w0 = w1;
+    }
+    ctx->last_kernel_ms = decode_ms + extract_ms;
+    if (frames_out)
+        for (uint32_t w = 0; w < n_windows; w++) frames_out[w] = plans[w].want;
+    return SEA_B200_OK;
 }
 
 // ------------------------------------------------------------------------------------------------ encode entry points

@@ -10,6 +10,7 @@
 #include <vector>
 
 #include "../../include/sea_b200.h"
+#include "sea_format.h"
 
 // capi.cu (not part of the public header): the decoder.rs:21 scale_factor_bits consistency check over a run of chunks
 extern "C" __attribute__((visibility("hidden"))) int sea_b200_internal_check_sf_bits(sea_b200_decoder *dec, const uint8_t *chunks, uint64_t len, uint64_t stride);
@@ -61,30 +62,22 @@ int sea_b200_decode_range(sea_b200_ctx *ctx, const uint8_t *sea, uint64_t len, u
     if (rc) return rc;
     if (sample_rate) *sample_rate = h.sample_rate;
     if (channels) *channels = h.channels;
-    uint64_t body = SEA_B200_FILE_HEADER_BYTES;
-    if (flags & SEA_B200_RANGE_SKIP_METADATA) body += h.metadata_size;  // what file.rs:53-54 meant to do
-    if (body > len) return SEA_B200_ERR_IO;
-    const uint64_t N = h.frames_per_chunk, avail_chunks = (len - body + h.chunk_size - 1) / h.chunk_size;
-    // frames the file can deliver: total_frames (clamped to the chunks present, file.rs:186-188) or, streaming, whole chunks
-    uint64_t file_frames = h.total_frames ? std::min<uint64_t>(h.total_frames, avail_chunks * N) : (len - body) / h.chunk_size * N;
-    if (first_frame >= file_frames || n_frames == 0) return SEA_B200_OK;
-    const uint64_t end_frame = std::min(file_frames, first_frame + n_frames);
-    const uint64_t k0 = first_frame / N, k1 = (end_frame + N - 1) / N;  // chunk k starts at body + k*chunk_size (file.rs:185)
-    const uint64_t want = (end_frame - first_frame) * h.channels;
+    sea::RangePlan r;
+    if ((rc = sea::plan_range(h, len, first_frame, n_frames, flags & SEA_B200_RANGE_SKIP_METADATA, &r)) != SEA_B200_OK) return rc;
+    if (r.want == 0) return SEA_B200_OK;
+    const uint64_t want = r.want * h.channels;
     if (!pcm) {  // size query (c/sea.h:209-211 pattern)
         *n_samples = want;
         return SEA_B200_OK;
     }
     if (want > pcm_cap_samples) return SEA_B200_ERR_CAPACITY;
-    const uint64_t b0 = body + k0 * h.chunk_size, b1 = std::min<uint64_t>(len, body + k1 * h.chunk_size);
-    // whole chunks only: a chunk's section layout depends on its own frame count (chunk.rs:105-113), so the sub-file keeps
-    // every covered chunk at its true length and the requested frames are cut out afterwards
-    const uint64_t sub_frames = std::min(file_frames, k1 * N) - k0 * N;
+    const uint64_t sub_frames = r.sub_frames;
     if (sub_frames > 0xffffffffull) return SEA_B200_ERR_TOO_MANY_FRAMES;
-    std::vector<uint8_t> file(SEA_B200_FILE_HEADER_BYTES + (b1 - b0));
+    // the sub-file keeps every covered chunk at its true length (see plan_range); the requested frames are cut out afterwards
+    std::vector<uint8_t> file(SEA_B200_FILE_HEADER_BYTES + (r.b1 - r.b0));
     write_header(file.data(), h, (uint32_t)sub_frames);
-    memcpy(file.data() + SEA_B200_FILE_HEADER_BYTES, sea + b0, b1 - b0);
-    const uint64_t skip = (first_frame - k0 * N) * h.channels;
+    memcpy(file.data() + SEA_B200_FILE_HEADER_BYTES, sea + r.b0, r.b1 - r.b0);
+    const uint64_t skip = r.skip * h.channels;
     if (skip == 0 && want == sub_frames * h.channels) {
         uint64_t got = 0;
         rc = sea_b200_decode(ctx, file.data(), file.size(), pcm, pcm_cap_samples, &got, nullptr, nullptr);

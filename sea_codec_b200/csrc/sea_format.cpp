@@ -6,6 +6,8 @@
 #include <math.h>
 #include <string.h>
 
+#include <algorithm>
+
 namespace sea {
 
 static inline uint32_t rd_u16(const uint8_t *p) { return (uint32_t)p[0] | ((uint32_t)p[1] << 8); }
@@ -44,6 +46,29 @@ void write_file_header(uint8_t *p, uint8_t channels, uint16_t chunk_size, uint16
     for (int i = 0; i < 4; i++) p[10 + i] = (uint8_t)(sample_rate >> (8 * i));
     for (int i = 0; i < 4; i++) p[14 + i] = (uint8_t)(total_frames >> (8 * i));
     memset(p + 18, 0, 4);
+}
+
+int plan_range(const sea_b200_header &h, uint64_t len, uint64_t first_frame, uint64_t n_frames, bool skip_metadata, RangePlan *p)
+{
+    memset(p, 0, sizeof(*p));
+    p->body = kFileHeaderBytes;
+    if (skip_metadata) p->body += h.metadata_size;  // what file.rs:53-54 meant to do
+    if (p->body > len) return SEA_B200_ERR_IO;
+    const uint64_t N = h.frames_per_chunk, avail_chunks = (len - p->body + h.chunk_size - 1) / h.chunk_size;
+    // total_frames clamped to the chunks present (file.rs:186-188) or, streaming, whole chunks
+    p->file_frames = h.total_frames ? std::min<uint64_t>(h.total_frames, avail_chunks * N) : (len - p->body) / h.chunk_size * N;
+    if (first_frame >= p->file_frames || n_frames == 0) return SEA_B200_OK;
+    const uint64_t end_frame = std::min(p->file_frames, first_frame + n_frames);
+    p->k0 = first_frame / N;
+    p->k1 = (end_frame + N - 1) / N;
+    p->b0 = p->body + p->k0 * h.chunk_size;
+    p->b1 = std::min<uint64_t>(len, p->body + p->k1 * h.chunk_size);
+    // whole chunks only: a chunk's section layout depends on its own frame count (chunk.rs:105-113), so every covered chunk is
+    // decoded at its true length and the requested frames are cut out afterwards
+    p->sub_frames = std::min(p->file_frames, p->k1 * N) - p->k0 * N;
+    p->skip = first_frame - p->k0 * N;
+    p->want = end_frame - first_frame;
+    return SEA_B200_OK;
 }
 
 // encoder_vbr.rs:40-63, evaluated in f32 in source order.

@@ -16,6 +16,20 @@ int parse_file_header(const uint8_t *p, uint64_t len, sea_b200_header *h);
 void write_file_header(uint8_t *p, uint8_t channels, uint16_t chunk_size, uint16_t frames_per_chunk, uint32_t sample_rate,
                        uint32_t total_frames);
 
+// ---- random access: which chunks cover frames [first_frame, first_frame + n_frames) of a file -------------
+// Shared by sea_b200_decode_range and sea_b200_decode_windows_device, so that a window holds exactly what decode_range returns.
+struct RangePlan {
+    uint64_t body;         // byte offset of chunk 0 (22, or 22 + metadata_size with the metadata skip)
+    uint64_t file_frames;  // frames the file can deliver: total_frames clamped to the chunks present, or, streaming, whole chunks
+    uint64_t k0, k1;       // covering chunks [k0, k1); chunk k starts at body + k * chunk_size (file.rs:185)
+    uint64_t b0, b1;       // their bytes [b0, b1) in the file (b1 clamped to its length)
+    uint64_t sub_frames;   // frames of the covering chunks: whole chunks, or up to the file's end
+    uint64_t skip;         // frames of chunk k0 before first_frame
+    uint64_t want;         // frames of the range the file has (0: nothing to decode)
+};
+// SEA_B200_ERR_IO when the body starts past the file's end; otherwise OK (want == 0 for an empty range).
+int plan_range(const sea_b200_header &h, uint64_t len, uint64_t first_frame, uint64_t n_frames, bool skip_metadata, RangePlan *p);
+
 // ---- settings ------------------------------------------------------------------------------------------
 // Resolved, validated view of EncoderSettings for one (channels) configuration.
 struct EncodePlan {

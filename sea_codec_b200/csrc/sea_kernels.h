@@ -87,6 +87,21 @@ inline uint32_t pick_cta_warps(uint64_t total_chunks, uint32_t chunks_per_warp, 
     return warps;
 }
 
+// Window cut (window_kernels.cu): one descriptor per window of sea_b200_decode_windows_device.  The covering chunks were decoded
+// into a scratch buffer; the kernel writes the slot: `real` frames from scratch, then zeros up to `frames`.
+struct WinDesc {
+    uint64_t src;       // scratch sample offset of the window's first frame (covering range start + skip * channels)
+    uint64_t dst;       // element offset of the slot in the output
+    uint32_t real;      // frames copied from scratch
+    uint32_t frames;    // frames of the slot
+    uint32_t channels;
+    uint32_t pad;
+};
+// planar_f32 = false: int16 interleaved [frames][channels]; true: float32 planar [channels][frames], sample / 32768.
+// max_slot_samples: the largest frames * channels of the launch (sizes the grid).
+cudaError_t launch_window_extract(const int16_t *d_scratch, void *d_out, const WinDesc *d_desc, uint32_t n_windows, uint64_t max_slot_samples,
+                                  bool planar_f32, cudaStream_t stream);
+
 // ---- encode ------------------------------------------------------------------------------------------------
 struct EncStream {
     uint64_t pcm_off;   // sample offset of the stream's PCM
