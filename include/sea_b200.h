@@ -230,6 +230,38 @@ int sea_b200_decode_windows_device(sea_b200_ctx *ctx, uint32_t n_streams, const 
                                    const uint32_t *window_stream, const uint64_t *first_frames, const uint32_t *n_frames,
                                    uint32_t flags, void *d_out, const uint64_t *out_offsets, uint64_t *frames_out);
 
+/* A registered corpus: .sea streams resident in device memory, checked once, then decoded in fixed-length windows from indices
+ * that live on the device, stream-ordered and without host synchronisation (a training loader's crops, inside a CUDA graph). */
+typedef struct sea_b200_corpus sea_b200_corpus;
+/* Registers n_streams .sea streams resident in device memory of ctx's GPU, described as for sea_b200_decode_windows_device
+ * (d_sea + host sea_offsets / sea_lens, n_streams * 22 header bytes on the host).  flags: 0 or SEA_B200_RANGE_SKIP_METADATA
+ * (fixed for the corpus).  All streams must have the same channel count.  Every chunk any window could cover is validated
+ * here, once: a stream the reference could not decode is rejected with the code decode_range would return for it, and
+ * last_error names the stream and the chunk.  d_sea must stay valid and unchanged for the life of the corpus, and the corpus
+ * must be destroyed before ctx.  Synchronous; not capturable. */
+int sea_b200_corpus_create(sea_b200_ctx *ctx, uint32_t n_streams, const uint8_t *d_sea, const uint64_t *sea_offsets,
+                           const uint64_t *sea_lens, const uint8_t *headers, uint32_t flags, sea_b200_corpus **corpus);
+void sea_b200_corpus_destroy(sea_b200_corpus *corpus); /* waits for work of the corpus still in flight */
+/* channels, and per stream the frames a window can draw from (stream_frames: n_streams entries, or NULL); route: 0 generic,
+ * 1 fast (informational; SEA_B200_CORPUS_ROUTE=generic|fast pins it at create, for tests). */
+int sea_b200_corpus_info(const sea_b200_corpus *corpus, uint32_t *channels, uint64_t *stream_frames, uint32_t *route);
+/* n_windows windows of window_frames frames each.  Window w = frames [d_first_frames[w], + window_frames) of stream
+ * d_window_stream[w]; both arrays are in DEVICE memory.  Slot w is dense in d_out:
+ *   default:                    int16   [n_windows][window_frames][channels]
+ *   SEA_B200_WINDOW_F32_PLANAR: float32 [n_windows][channels][window_frames]
+ * Slot w equals decode_windows_device's slot for (stream, first, window_frames) with the corpus's metadata flag: what
+ * decode_range returns, then zeros (a first frame at or past the stream's end, including any huge value, gives an all-zero
+ * slot).  d_frames_out[w] (device, nullable) equals its frames_out.  A stream index >= n_streams zero-fills the slot, writes
+ * frames_out 0 and stores SEA_B200_ERR_INVALID_PARAMETERS into *d_status when *d_status is 0 (first error wins; the call never
+ * clears it).  Bytes of d_out outside the slots are never written.
+ * Stream-ordered on the context's current stream: no host synchronisation, no allocation, no host<->device copy, so the call
+ * can be captured in a CUDA graph and replayed with new indices written in place.  For the same reason it does not update
+ * sea_b200_last_kernel_ms.  Host-checkable errors (NULL pointers, unknown flag bits, misaligned d_out) return before anything
+ * is enqueued; n_windows == 0 or window_frames == 0 enqueues nothing. */
+int sea_b200_corpus_decode_windows_async(sea_b200_corpus *corpus, uint32_t n_windows, const uint32_t *d_window_stream,
+                                         const uint64_t *d_first_frames, uint32_t window_frames, uint32_t flags, void *d_out,
+                                         uint32_t *d_frames_out, int32_t *d_status);
+
 /* ---------------------------------------------------------------- the reference's existing foreign surfaces */
 
 /* src/wasm_api.rs:32-111 (wasm_sea_encode / wasm_sea_decode / allocate / deallocate / setup) with the same argument lists,

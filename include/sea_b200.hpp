@@ -70,6 +70,44 @@ private:
     sea_b200_ctx *ctx_ = nullptr;
 };
 
+// A registered corpus (sea_b200_corpus_*): device-resident streams checked once, then decoded in fixed-length windows from device-side
+// indices on the context's stream, without host synchronisation (CUDA-graph capturable).  Destroy it before its Context.
+class Corpus {
+public:
+    Corpus(Context &ctx, uint32_t n_streams, const uint8_t *d_sea, const uint64_t *sea_offsets, const uint64_t *sea_lens,
+           const uint8_t *headers, bool skip_metadata = false)
+        : ctx_(&ctx)
+    {
+        ctx.check(sea_b200_corpus_create(ctx.get(), n_streams, d_sea, sea_offsets, sea_lens, headers,
+                                         skip_metadata ? SEA_B200_RANGE_SKIP_METADATA : 0u, &corpus_));
+        uint32_t route = 0;
+        stream_frames_.resize(n_streams);
+        ctx.check(sea_b200_corpus_info(corpus_, &channels_, stream_frames_.data(), &route));
+        fast_ = route == 1;
+    }
+    ~Corpus() { sea_b200_corpus_destroy(corpus_); }
+    Corpus(const Corpus &) = delete;
+    Corpus &operator=(const Corpus &) = delete;
+    sea_b200_corpus *get() const { return corpus_; }
+    uint32_t channels() const { return channels_; }
+    bool fast_route() const { return fast_; }
+    const std::vector<uint64_t> &stream_frames() const { return stream_frames_; }
+    // see sea_b200_corpus_decode_windows_async; flags: 0 or SEA_B200_WINDOW_F32_PLANAR
+    void decode_windows_async(uint32_t n_windows, const uint32_t *d_window_stream, const uint64_t *d_first_frames, uint32_t window_frames,
+                              uint32_t flags, void *d_out, uint32_t *d_frames_out, int32_t *d_status) const
+    {
+        ctx_->check(sea_b200_corpus_decode_windows_async(corpus_, n_windows, d_window_stream, d_first_frames, window_frames, flags, d_out,
+                                                         d_frames_out, d_status));
+    }
+
+private:
+    Context *ctx_;
+    sea_b200_corpus *corpus_ = nullptr;
+    uint32_t channels_ = 0;
+    bool fast_ = false;
+    std::vector<uint64_t> stream_frames_;
+};
+
 // Every GPU of the box behind one handle (sea_b200_multi, SURVEY 8e): batch calls shard the streams over the GPUs in-process --
 // one context and one host thread per GPU, nothing exchanged between them -- and report per-GPU counts.
 class MultiContext {

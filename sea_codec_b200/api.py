@@ -138,6 +138,12 @@ SYMBOLS = {
                                         _u64p, _u32p, _u32p]),
     "sea_b200_decode_windows_device": (C.c_int, [C.c_void_p, C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32,
                                                  C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "sea_b200_corpus_create": (C.c_int, [C.c_void_p, C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32,
+                                         C.POINTER(C.c_void_p)]),
+    "sea_b200_corpus_destroy": (None, [C.c_void_p]),
+    "sea_b200_corpus_info": (C.c_int, [C.c_void_p, _u32p, C.c_void_p, _u32p]),
+    "sea_b200_corpus_decode_windows_async": (C.c_int, [C.c_void_p, C.c_uint32, C.c_void_p, C.c_void_p, C.c_uint32, C.c_uint32,
+                                                       C.c_void_p, C.c_void_p, C.c_void_p]),
     "sea_b200_wasm_setup": (None, []),
     "sea_b200_wasm_sea_encode": (C.c_size_t, [C.c_void_p, C.c_size_t, C.c_uint32, C.c_uint32, C.c_float, C.c_bool, C.c_void_p, C.c_size_t]),
     "sea_b200_wasm_sea_decode": (C.c_size_t, [C.c_void_p, C.c_size_t, C.c_void_p, C.c_size_t, _u32p, _u32p]),
@@ -422,6 +428,112 @@ class Context:
                                                            hd.ctypes.data, ws.size, ws.ctypes.data, ff.ctypes.data, nf.ctypes.data, flags,
                                                            C.c_void_p(d_out), oo.ctypes.data, out.ctypes.data))
         return out
+
+    def corpus(self, buf, sea_offsets, sea_lens, headers: np.ndarray, skip_metadata: bool = False) -> "Corpus":
+        """Registers the .sea streams held in `buf` (a uint8 CUDA tensor; streams described as for decode_windows_device) for
+        Corpus.decode_windows.  Every chunk a window can cover is validated here, once."""
+        return Corpus(self, buf, sea_offsets, sea_lens, headers, skip_metadata)
+
+
+class Corpus:
+    """A registered corpus (sea_b200_corpus): fixed-length windows decoded from device-side indices on the current torch stream,
+    with no host synchronisation, so the call can sit inside torch.cuda.graph(...).  Keeps `buf` and its Context alive.  A loader
+    draws valid starts on the device, e.g. (torch.rand(n, device=dev) * (stream_frames_cuda[s] - W + 1)).long()."""
+
+    def __init__(self, ctx: Context, buf, sea_offsets, sea_lens, headers: np.ndarray, skip_metadata: bool = False):
+        import torch
+
+        if not (isinstance(buf, torch.Tensor) and buf.is_cuda and buf.dtype == torch.uint8 and buf.is_contiguous()):
+            raise SeaError(ERR_INVALID_PARAMETERS, "buf must be a contiguous uint8 CUDA tensor")
+        so, sl = _u64(sea_offsets), _u64(sea_lens)
+        hd = np.ascontiguousarray(headers, dtype=np.uint8)
+        if so.size != sl.size or hd.size < so.size * 22:
+            raise SeaError(ERR_INVALID_PARAMETERS, "stream arrays differ in length")
+        if so.size and int(np.max(so + sl)) > buf.numel():
+            raise SeaError(ERR_INVALID_PARAMETERS, "a stream runs past the end of buf")
+        self._h = C.c_void_p()
+        self._ctx, self._L, self._buf = ctx, ctx._L, buf
+        self.device = torch.device("cuda", ctx.device)
+        # bind the context to torch's stream now: dropping its own stream synchronises, which a later capture must not do
+        ctx.set_stream(torch.cuda.current_stream(self.device).cuda_stream)
+        ctx._check(self._L.sea_b200_corpus_create(ctx._h, so.size, C.c_void_p(buf.data_ptr()), so.ctypes.data, sl.ctypes.data,
+                                                  hd.ctypes.data, RANGE_SKIP_METADATA if skip_metadata else 0, C.byref(self._h)))
+        ch, route = C.c_uint32(0), C.c_uint32(0)
+        self.stream_frames = np.zeros(so.size, dtype=np.uint64)
+        ctx._check(self._L.sea_b200_corpus_info(self._h, C.byref(ch), self.stream_frames.ctypes.data, C.byref(route)))
+        self.n_streams = int(so.size)
+        self.channels = int(ch.value)
+        self.route = "fast" if route.value else "generic"
+        self.stream_frames_cuda = torch.from_numpy(self.stream_frames.astype(np.int64)).to(self.device)
+        self._status = torch.zeros(1, dtype=torch.int32, device=self.device)
+
+    def close(self):
+        if getattr(self, "_h", None) and self._h.value:
+            self._L.sea_b200_corpus_destroy(self._h)
+            self._h = C.c_void_p()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    @property
+    def status(self):
+        """The persistent int32 status tensor decode_windows uses by default (0, or the first error's SeaError code)."""
+        return self._status
+
+    def decode_windows(self, stream_idx, first_frames, window_frames: int, *, float32_planar: bool = False, out=None,
+                       frames_out=None, status=None):
+        """Windows [first_frames[w], + window_frames) of streams stream_idx[w] (int32 or int64 CUDA tensors) into `out`: int16
+        [n, window_frames, channels], or with float32_planar float32 [n, channels, window_frames] = sample / 32768 (allocated when
+        not given; a given `out` is any contiguous CUDA tensor of that dtype and element count).  Each slot holds what decode_range
+        returns for its window, then zeros; frames_out (int32 CUDA tensor of n, optional) gets the real frames per window.  A
+        stream index out of range zero-fills its slot and sets `status` (default: the corpus's own, see check()).  Enqueued on
+        torch.cuda.current_stream() without host synchronisation or allocation beyond `out`."""
+        import torch
+
+        n = stream_idx.numel()
+        if first_frames.numel() != n:
+            raise SeaError(ERR_INVALID_PARAMETERS, "stream_idx and first_frames differ in length")
+        for t in (stream_idx, first_frames):
+            if not (t.is_cuda and t.dtype in (torch.int32, torch.int64)):
+                raise SeaError(ERR_INVALID_PARAMETERS, "indices must be int32 or int64 CUDA tensors")
+        W, ch = int(window_frames), self.channels
+        if not 0 <= W < 2**32:
+            raise SeaError(ERR_INVALID_PARAMETERS, "window_frames must fit 32 bits")
+        # uint32 stream indices: a negative or too large index stays out of range (-1 -> 0xffffffff)
+        si = stream_idx.reshape(-1)
+        if si.dtype == torch.int64:
+            si = si.clamp(-1, 2**31 - 1).to(torch.int32)
+        si = si.contiguous()
+        ff = first_frames.reshape(-1).to(torch.int64).contiguous()  # read as uint64: negative starts lie past every stream's end
+        dtype = torch.float32 if float32_planar else torch.int16
+        if out is None:
+            out = torch.empty((n, ch, W) if float32_planar else (n, W, ch), dtype=dtype, device=self.device)
+        elif not (out.is_cuda and out.dtype == dtype and out.is_contiguous() and out.numel() == n * W * ch):
+            raise SeaError(ERR_INVALID_PARAMETERS, f"out must be a contiguous {dtype} CUDA tensor of {n * W * ch} elements")
+        fo = 0
+        if frames_out is not None:
+            if not (frames_out.is_cuda and frames_out.dtype == torch.int32 and frames_out.is_contiguous() and frames_out.numel() == n):
+                raise SeaError(ERR_INVALID_PARAMETERS, "frames_out must be a contiguous int32 CUDA tensor of n elements")
+            fo = frames_out.data_ptr()
+        st = self._status if status is None else status
+        if not (st.is_cuda and st.dtype == torch.int32 and st.numel() >= 1):
+            raise SeaError(ERR_INVALID_PARAMETERS, "status must be an int32 CUDA tensor")
+        self._ctx.set_stream(torch.cuda.current_stream(self.device).cuda_stream)
+        flags = WINDOW_F32_PLANAR if float32_planar else 0
+        self._ctx._check(self._L.sea_b200_corpus_decode_windows_async(self._h, n, C.c_void_p(si.data_ptr()), C.c_void_p(ff.data_ptr()),
+                                                                      W, flags, C.c_void_p(out.data_ptr()), C.c_void_p(fo),
+                                                                      C.c_void_p(st.data_ptr())))
+        return out
+
+    def check(self):
+        """Synchronises with the corpus's status tensor, raises SeaError if a call stored an error there, and clears it."""
+        code = int(self._status.item())
+        if code:
+            self._status.zero_()
+            raise SeaError(code, "a window named a stream index out of range")
 
 
 class MultiContext:

@@ -10,8 +10,8 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libsea_b200.so")
-SOURCES = ["capi.cu", "capi_ext.cu", "capi_multi.cpp", "decode_kernels.cu", "decode_fast.cu", "decode_fast_mono.cu", "decode_vbr.cu", "decode_mc.cu", "decode_mc_odd.cu", "decode_latency.cu", "encode_kernels.cu", "misc_kernels.cu", "window_kernels.cu", "sea_format.cpp"]
-HEADERS = ["sea_common.cuh", "sea_device.cuh", "decode_mc.cuh", "decode_fast.cuh", "sea_format.h", "sea_kernels.h", os.path.join("..", "..", "include", "sea_b200.h")]
+SOURCES = ["capi.cu", "capi_ext.cu", "capi_multi.cpp", "decode_kernels.cu", "decode_fast.cu", "decode_fast_mono.cu", "decode_vbr.cu", "decode_mc.cu", "decode_mc_odd.cu", "decode_latency.cu", "encode_kernels.cu", "misc_kernels.cu", "window_kernels.cu", "corpus_kernels.cu", "sea_format.cpp"]
+HEADERS = ["sea_common.cuh", "sea_device.cuh", "decode_chain.cuh", "decode_mc.cuh", "decode_fast.cuh", "sea_format.h", "sea_kernels.h", os.path.join("..", "..", "include", "sea_b200.h")]
 
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",

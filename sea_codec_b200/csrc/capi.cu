@@ -1336,6 +1336,192 @@ int sea_b200_decode_windows_device(sea_b200_ctx *ctx, uint32_t n_streams, const 
     return SEA_B200_OK;
 }
 
+// ------------------------------------------------------------------------------------------------ registered corpus
+
+}  // extern "C"
+
+struct sea_b200_corpus {
+    sea_b200_ctx *ctx;
+    uint32_t n_streams, channels;
+    bool fast;
+    const uint8_t *d_sea;
+    uint64_t sea_len;                    // readable bytes from d_sea: the end of the furthest stream
+    CorpusStream *d_streams = nullptr;
+    std::vector<uint64_t> stream_frames;
+    uint32_t N_min, s, b;                // smallest frames_per_chunk; the fast route's header fields
+};
+
+extern "C" {
+
+// The stream table and every chunk a window can cover are checked here, once (corpus_validate_kernel): the async call then has no
+// malformed-chunk path, no error word to read back and no fallback, which is what lets it run without a host synchronisation.
+int sea_b200_corpus_create(sea_b200_ctx *ctx, uint32_t n_streams, const uint8_t *d_sea, const uint64_t *sea_offsets,
+                           const uint64_t *sea_lens, const uint8_t *headers, uint32_t flags, sea_b200_corpus **corpus)
+{
+    if (!ctx || !corpus) return SEA_B200_ERR_INVALID_PARAMETERS;
+    *corpus = nullptr;
+    if (!d_sea || !sea_offsets || !sea_lens || !headers || n_streams == 0)
+        return fail(ctx, SEA_B200_ERR_INVALID_PARAMETERS, "a corpus needs at least one stream and every pointer");
+    if (flags & ~SEA_B200_RANGE_SKIP_METADATA) return fail(ctx, SEA_B200_ERR_INVALID_PARAMETERS, "unknown flag bits");
+    int force = -1;  // SEA_B200_CORPUS_ROUTE = generic / fast pins the route (tests)
+    if (const char *env = getenv("SEA_B200_CORPUS_ROUTE")) {
+        if (!strcmp(env, "generic")) force = 0;
+        else if (!strcmp(env, "fast")) force = 1;
+        else return fail(ctx, SEA_B200_ERR_INVALID_PARAMETERS, "SEA_B200_CORPUS_ROUTE must be generic or fast");
+    }
+    std::vector<CorpusStream> table(n_streams);
+    std::vector<uint64_t> frames(n_streams);
+    uint32_t channels = 0, N_min = 0xffffffffu;
+    bool uniform = true;
+    uint64_t chunks = 0, sea_len = 0;
+    for (uint32_t i = 0; i < n_streams; i++) {
+        const uint64_t len = sea_lens[i];
+        sea_b200_header h;
+        int rc = parse_file_header(headers + (size_t)i * kFileHeaderBytes, len < 22 ? len : 22, &h);
+        if (rc) return fail(ctx, rc, "stream " + std::to_string(i) + ": bad .sea header (file.rs:40-72)");
+        if (i == 0) channels = h.channels;
+        if (h.channels != channels)
+            return fail(ctx, SEA_B200_ERR_INVALID_PARAMETERS, "stream " + std::to_string(i) + " has " + std::to_string(h.channels) +
+                                                                  " channels, stream 0 has " + std::to_string(channels));
+        RangePlan rp;
+        rc = plan_range(h, len, 0, 0, flags & SEA_B200_RANGE_SKIP_METADATA, &rp);
+        if (rc) return fail(ctx, rc, "stream " + std::to_string(i) + ": metadata runs past the end of the stream");
+        if (rp.file_frames > 0xffffffffull)
+            return fail(ctx, SEA_B200_ERR_TOO_MANY_FRAMES, "stream " + std::to_string(i) + ": longer than 2^32 frames");
+        CorpusStream &t = table[i];
+        memset(&t, 0, sizeof(t));
+        t.body = sea_offsets[i] + rp.body;
+        t.len = len - rp.body;
+        t.file_frames = rp.file_frames;
+        t.chunk_begin = chunks;
+        t.chunk_size = h.chunk_size;
+        t.N = h.frames_per_chunk;
+        t.n_chunks = (uint32_t)((rp.file_frames + t.N - 1) / t.N);
+        chunks += t.n_chunks;
+        frames[i] = rp.file_frames;
+        N_min = std::min(N_min, t.N);
+        if (t.chunk_size != table[0].chunk_size || t.N != table[0].N) uniform = false;
+        sea_len = std::max(sea_len, sea_offsets[i] + len);
+    }
+    CU(cudaSetDevice(ctx->device));
+    // every chunk is compared with the first chunk of the first stream that has one
+    uint32_t ref_word = 0;
+    for (uint32_t i = 0; i < n_streams; i++)
+        if (table[i].n_chunks) {
+            uint8_t b[4] = {0, 0, 0, 0};
+            CU(cudaMemcpy(b, d_sea + table[i].body, std::min<uint64_t>(4, table[i].len), cudaMemcpyDeviceToHost));
+            ref_word = (uint32_t)b[0] | ((uint32_t)b[1] << 8) | ((uint32_t)b[2] << 16) | ((uint32_t)b[3] << 24);
+            break;
+        }
+
+    sea_b200_corpus *c = new sea_b200_corpus();
+    c->ctx = ctx;
+    auto bail = [&](int rc) {
+        sea_b200_corpus_destroy(c);
+        return rc;
+    };
+    cudaError_t e = cudaMalloc(&c->d_streams, sizeof(CorpusStream) * n_streams);
+    if (e != cudaSuccess) return bail(cuda_fail(ctx, e, "cudaMalloc(corpus stream table)"));
+    e = cudaMemcpy(c->d_streams, table.data(), sizeof(CorpusStream) * n_streams, cudaMemcpyHostToDevice);
+    if (e != cudaSuccess) return bail(cuda_fail(ctx, e, "cudaMemcpy(corpus stream table)"));
+    struct { unsigned long long first_bad; uint32_t mixed, pad; } res = {~0ull, 0u, 0u};
+    void *d_res = nullptr;
+    if ((e = cudaMalloc(&d_res, sizeof(res))) != cudaSuccess) return bail(cuda_fail(ctx, e, "cudaMalloc(corpus check words)"));
+    e = cudaMemcpyAsync(d_res, &res, sizeof(res), cudaMemcpyHostToDevice, ctx->stream);
+    if (e == cudaSuccess)
+        e = launch_corpus_validate(d_sea, c->d_streams, n_streams, chunks, channels, ref_word, static_cast<unsigned long long *>(d_res),
+                                   reinterpret_cast<uint32_t *>(static_cast<uint8_t *>(d_res) + 8), ctx->stream);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(&res, d_res, sizeof(res), cudaMemcpyDeviceToHost, ctx->stream);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
+    cudaFree(d_res);
+    if (e != cudaSuccess) return bail(cuda_fail(ctx, e, "corpus validation"));
+    ctx->launches++;
+    if (res.first_bad != ~0ull) {
+        const uint64_t g = res.first_bad >> 2;
+        uint32_t i = 0;
+        while (i + 1 < n_streams && table[i + 1].chunk_begin <= g) i++;
+        const int rc = map_dev_error(ctx, (int)(res.first_bad & 3u));
+        ctx->last_error = "stream " + std::to_string(i) + ", chunk " + std::to_string(g - table[i].chunk_begin) + ": " + ctx->last_error;
+        return bail(rc);
+    }
+    const uint32_t type = ref_word & 0xffu, s = (ref_word >> 12) & 15u, b = (ref_word >> 8) & 15u, F = (ref_word >> 16) & 0xffu;
+    const bool qualifies = chunks > 0 && uniform && !res.mixed && corpus_fast_supported(channels, s, b, F, type == 2u);
+    if (force == 1 && !qualifies)
+        return bail(fail(ctx, SEA_B200_ERR_INVALID_PARAMETERS,
+                         "SEA_B200_CORPUS_ROUTE=fast: the corpus does not qualify (it needs uniform CBR chunks, 1 or 2 channels, "
+                         "scale_factor_frames 20, scale_factor_bits <= 5)"));
+    c->fast = force >= 0 ? force == 1 : qualifies;
+    if (c->fast && (e = corpus_fast_prepare(channels, s, b)) != cudaSuccess) return bail(cuda_fail(ctx, e, "corpus_fast_prepare"));
+    c->n_streams = n_streams;
+    c->channels = channels;
+    c->d_sea = d_sea;
+    c->sea_len = sea_len;
+    c->stream_frames = std::move(frames);
+    c->N_min = N_min == 0xffffffffu ? 1u : N_min;
+    c->s = s;
+    c->b = b;
+    *corpus = c;
+    return SEA_B200_OK;
+}
+
+void sea_b200_corpus_destroy(sea_b200_corpus *corpus)
+{
+    if (!corpus) return;
+    cudaSetDevice(corpus->ctx->device);
+    if (corpus->ctx->stream) cudaStreamSynchronize(corpus->ctx->stream);
+    if (corpus->d_streams) cudaFree(corpus->d_streams);  // also waits for the corpus's work on any other stream
+    delete corpus;
+}
+
+int sea_b200_corpus_info(const sea_b200_corpus *corpus, uint32_t *channels, uint64_t *stream_frames, uint32_t *route)
+{
+    if (!corpus) return SEA_B200_ERR_INVALID_PARAMETERS;
+    if (channels) *channels = corpus->channels;
+    if (stream_frames) memcpy(stream_frames, corpus->stream_frames.data(), sizeof(uint64_t) * corpus->n_streams);
+    if (route) *route = corpus->fast ? 1u : 0u;
+    return SEA_B200_OK;
+}
+
+// Enqueues one kernel on the context's stream and nothing else: no allocation, no copy, no synchronisation (graph-capturable).
+int sea_b200_corpus_decode_windows_async(sea_b200_corpus *corpus, uint32_t n_windows, const uint32_t *d_window_stream,
+                                         const uint64_t *d_first_frames, uint32_t window_frames, uint32_t flags, void *d_out,
+                                         uint32_t *d_frames_out, int32_t *d_status)
+{
+    if (!corpus) return SEA_B200_ERR_INVALID_PARAMETERS;
+    sea_b200_ctx *ctx = corpus->ctx;
+    if (flags & ~SEA_B200_WINDOW_F32_PLANAR) return fail(ctx, SEA_B200_ERR_INVALID_PARAMETERS, "unknown flag bits");
+    if (n_windows == 0 || window_frames == 0) return SEA_B200_OK;
+    if (!d_window_stream || !d_first_frames || !d_out || !d_status) return fail(ctx, SEA_B200_ERR_INVALID_PARAMETERS, "NULL pointer");
+    const bool planar = flags & SEA_B200_WINDOW_F32_PLANAR;
+    if (reinterpret_cast<uintptr_t>(d_out) % (planar ? sizeof(float) : sizeof(int16_t)))
+        return fail(ctx, SEA_B200_ERR_INVALID_PARAMETERS, "d_out is not aligned to its element type");
+    const uint64_t M = ((uint64_t)window_frames + corpus->N_min - 2u) / corpus->N_min + 1u;  // most chunks a window can touch
+    if ((uint64_t)n_windows * M * corpus->channels > (1ull << 38))
+        return fail(ctx, SEA_B200_ERR_INVALID_PARAMETERS, "too many windows x covering chunks for one launch");
+    CorpusLaunch p = {};
+    p.sea = corpus->d_sea;
+    p.sea_len = corpus->sea_len;
+    p.streams = corpus->d_streams;
+    p.n_streams = corpus->n_streams;
+    p.channels = corpus->channels;
+    p.win_stream = d_window_stream;
+    p.win_first = d_first_frames;
+    p.n_windows = n_windows;
+    p.W = window_frames;
+    p.M = (uint32_t)M;
+    p.planar = planar;
+    p.out = d_out;
+    p.frames_out = d_frames_out;
+    p.status = d_status;
+    p.N = corpus->N_min;
+    p.s = corpus->s;
+    p.b = corpus->b;
+    CU(cudaSetDevice(ctx->device));
+    CU(launch_corpus_windows(p, corpus->fast, ctx->tabs, ctx->stream));
+    ctx->launches++;
+    return SEA_B200_OK;
+}
+
 // ------------------------------------------------------------------------------------------------ encode entry points
 
 int sea_b200_encode_batch_device(sea_b200_ctx *ctx, uint32_t n_streams, const int16_t *d_pcm, const uint64_t *pcm_offsets,

@@ -9,24 +9,12 @@
 //   decode_staged_kernel   uniform batches with 1 or 2 channels: a warp owns 32/C consecutive chunks, stages
 //                          their packed residuals through shared memory with coalesced 128-bit loads, decodes
 //                          one chain per lane and stages the PCM back out for coalesced interleaved stores.
-#include "sea_device.cuh"
+#include "decode_chain.cuh"
 
 namespace sea {
 
 using namespace dev;
 
-
-// MSB-first field of n <= 8 bits at bit offset `bit` from p (bits.rs:42-46 semantics), p in global memory.
-__device__ __forceinline__ uint32_t get_bits_gmem(const uint8_t *p, uint64_t bit, uint32_t n)
-{
-    uint64_t byte = bit >> 3;
-    uint32_t sh = (uint32_t)bit & 7u;
-    uint32_t v = (uint32_t)__ldg(p + byte) << 8;
-    if (sh + n > 8u) v |= (uint32_t)__ldg(p + byte + 1);
-    return (v >> (16u - sh - n)) & ((1u << n) - 1u);
-}
-
-// stream lookup: last stream whose chain_begin <= id
 
 // ------------------------------------------------------------------------------------------------ generic
 
@@ -48,12 +36,9 @@ __global__ void __launch_bounds__(128) decode_generic_kernel(const uint8_t *__re
     uint32_t frames = st.total_frames - k * N;
     if (frames > N) frames = N;
 
-    if (take < 4u + 16u * C) return report(err, kDevDomain);  // slice index out of range in chunk.rs:81-101
-    const uint32_t type = ck[0], s = ck[1] >> 4, b = ck[1] & 15u, F = ck[2];
-    if (type != 1u && type != 2u) return report(err, kDevInvalidFrame);  // chunk.rs:81-85
-    if (b < 1u || b > 8u || s < 1u || s > 8u || F == 0u) return report(err, kDevDomain);
-    const bool vbr = type == 2u;
-
+    auto fail = [&](int code) { report(err, code); };
+    ChunkGeom g;
+    if (!chunk_head(ck, take, C, g, fail)) return;
     int32_t w[4], h[4];
     {
         const uint8_t *l = ck + 4u + 16u * c;  // lms.rs:80-94
@@ -65,45 +50,13 @@ __global__ void __launch_bounds__(128) decode_generic_kernel(const uint8_t *__re
     }
     int32_t sg[4];
     lms_signs(sg, h);
-    const uint32_t nblk = div_ceil_u32(frames, F), items = nblk * C;
-    const uint32_t sf_sec = 4u + 16u * C;
-    const uint32_t vbr_sec = sf_sec + div_ceil_u32(items * s, 8u);
-    const uint32_t res_sec = vbr_sec + (vbr ? div_ceil_u32(items * 2u, 8u) : 0u);
-    if (res_sec > take) return report(err, kDevDomain);
-    const uint64_t res_bits_avail = (uint64_t)(take - res_sec) * 8u;
-    if (!vbr && (uint64_t)frames * C * b > res_bits_avail) return report(err, kDevDomain);
+    if (!chunk_sections(take, C, frames, g, fail)) return;
 
-    const int32_t *tab = tabs.by_s[s];
     int16_t *out = pcm + st.pcm_off + (uint64_t)k * N * C + c;
-    uint64_t bitpos = 0;  // start of the current frame inside the residual section
-    for (uint32_t blk = 0; blk < nblk; blk++) {
-        const uint32_t sf = get_bits_gmem(ck + sf_sec, (uint64_t)(blk * C + c) * s, s);
-        uint32_t size = b, rowbits = C * b, prefix = c * b;
-        if (vbr) {  // chunk.rs:126-139: size = 2-bit code + residual_size - 1
-            rowbits = 0;
-            prefix = 0;
-            for (uint32_t cc = 0; cc < C; cc++) {
-                uint32_t sz = get_bits_gmem(ck + vbr_sec, (uint64_t)(blk * C + cc) * 2u, 2u) + b - 1u;
-                if (sz < 1u || sz > 8u) return report(err, kDevDomain);
-                if (cc < c) prefix += sz;
-                if (cc == c) size = sz;
-                rowbits += sz;
-            }
-        }
-        uint32_t nf = frames - blk * F;
-        if (nf > F) nf = F;
-        if (bitpos + (uint64_t)nf * rowbits > res_bits_avail) return report(err, kDevDomain);
-        const int32_t *row = tab + tab_dqt_off(s, size) + (sf << size);
-        for (uint32_t f = 0; f < nf; f++) {
-            const uint32_t code = get_bits_gmem(ck + res_sec, bitpos + prefix, size);
-            bitpos += rowbits;
-            const int32_t d = __ldg(row + code);
-            const int32_t y = clamp_i16((int32_t)((uint32_t)lms_predict(w, h) + (uint32_t)d));  // decoder.rs:38-45
-            *out = (int16_t)y;
-            out += C;
-            lms_update_sg(w, h, sg, y, d);
-        }
-    }
+    chain_blocks<true>(ck, g, C, c, frames, w, h, sg, tabs.by_s[g.s], [&](int32_t y) {
+        *out = (int16_t)y;
+        out += C;
+    }, fail);
 }
 
 cudaError_t launch_decode_generic(const uint8_t *d_sea, int16_t *d_pcm, const DecStream *d_streams, uint32_t n_streams,

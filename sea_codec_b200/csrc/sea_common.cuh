@@ -130,4 +130,20 @@ SEA_HD uint32_t quant_code(int32_t r, int32_t recip, uint32_t b)
 
 SEA_HD uint32_t div_ceil_u32(uint32_t a, uint32_t b) { return (a + b - 1u) / b; }
 
+// The window part of plan_range (sea_format.cpp) for a stream that delivers file_frames frames in chunks of N frames: frames
+// [first, first + n) start `skip` frames into chunk k0, and the stream has `want` of them.  Past the end (or n == 0): all zero, as
+// plan_range leaves them.  The corpus kernels evaluate it per window on the device.
+struct WindowPlan {
+    uint64_t k0, skip, want;
+};
+SEA_HD WindowPlan window_plan(uint64_t file_frames, uint32_t N, uint64_t first, uint64_t n)
+{
+    WindowPlan p = {0, 0, 0};
+    if (first >= file_frames || n == 0) return p;
+    p.k0 = first / N;
+    p.skip = first - p.k0 * N;
+    p.want = file_frames - first < n ? file_frames - first : n;
+    return p;
+}
+
 }  // namespace sea

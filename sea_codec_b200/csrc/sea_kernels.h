@@ -102,6 +102,45 @@ struct WinDesc {
 cudaError_t launch_window_extract(const int16_t *d_scratch, void *d_out, const WinDesc *d_desc, uint32_t n_windows, uint64_t max_slot_samples,
                                   bool planar_f32, cudaStream_t stream);
 
+// Registered corpus (corpus_kernels.cu, sea_b200_corpus_*): one entry per stream, made once at create.
+struct CorpusStream {
+    uint64_t body;         // byte offset of chunk 0 in the corpus buffer (plan_range's body + the stream's offset)
+    uint64_t len;          // bytes of the stream from body on
+    uint64_t file_frames;  // frames a window can draw from (plan_range's file_frames)
+    uint64_t chunk_begin;  // global index of the stream's chunk 0 among the chunks create validates
+    uint32_t chunk_size, N, n_chunks;  // n_chunks = ceil(file_frames / N): every chunk a window can cover
+    uint32_t pad;
+};
+// Create-time validation: every chunk of every stream at its true frame count, with decode_generic_kernel's checks.  *d_first_bad:
+// min over failing chunks of (global chunk << 2 | kDev code), left at ~0 when none fails.  *d_mixed: nonzero when some chunk's
+// 4-byte header word differs from ref_word.
+cudaError_t launch_corpus_validate(const uint8_t *d_sea, const CorpusStream *d_streams, uint32_t n_streams, uint64_t total_chunks,
+                                   uint32_t channels, uint32_t ref_word, unsigned long long *d_first_bad, uint32_t *d_mixed,
+                                   cudaStream_t stream);
+
+// One batch of fixed-length windows (sea_b200_corpus_decode_windows_async): work unit (window, covering-chunk slot j < M).
+struct CorpusLaunch {
+    const uint8_t *sea;
+    uint64_t sea_len;  // readable bytes from sea (the staged loads of the fast route stop there)
+    const CorpusStream *streams;
+    uint32_t n_streams, channels;
+    const uint32_t *win_stream;
+    const uint64_t *win_first;
+    uint32_t n_windows, W, M;
+    bool planar;
+    void *out;
+    uint32_t *frames_out;  // nullable
+    int32_t *status;
+    // fast route: the corpus's uniform geometry and header fields
+    uint32_t N, chunk_size, s, b;
+};
+// Fast route: CBR, 1 or 2 channels, scale_factor_frames 20, scale_factor_bits <= 5 (its dequant rows live in shared memory), one
+// chunk geometry for every stream.  corpus_fast_prepare (once, at create: not capturable) raises the shared-memory limit of its
+// kernels; launch_corpus_windows then only enqueues.
+bool corpus_fast_supported(uint32_t channels, uint32_t s, uint32_t b, uint32_t F, bool vbr);
+cudaError_t corpus_fast_prepare(uint32_t channels, uint32_t s, uint32_t b);
+cudaError_t launch_corpus_windows(const CorpusLaunch &p, bool fast, DevTables tabs, cudaStream_t stream);
+
 // ---- encode ------------------------------------------------------------------------------------------------
 struct EncStream {
     uint64_t pcm_off;   // sample offset of the stream's PCM

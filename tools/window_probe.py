@@ -9,7 +9,10 @@ Shapes: 4096 stereo 60 s 44.1 kHz CBR-3 streams, the same at VBR-3, and 256 eigh
 both output formats (int16 interleaved, float32 planar): windows/s and window Msamples/s from a host clock around the call (which
 ends in a device synchronise), the covered / window sample ratio from the covering-chunk arithmetic, decode and extract kernel ms
 (CUDA events, from the library's SEA_B200_TRACE lines), and next to it the full-stream decode_batch_device of the same streams.
-The card's name and power limit are read in the same run.
+The card's name and power limit are read in the same run.  "async" under each format: the registered-corpus form
+(Context.corpus + Corpus.decode_windows) on the same windows -- GPU ms per call from CUDA events around back-to-back calls, host
+enqueue us per call, graph-replay ms per call with one call captured, the route, and whether its slots and frames_out equal
+decode_windows_device's.
 """
 from __future__ import annotations
 
@@ -113,6 +116,7 @@ def shape(ctx, torch, name, n_streams, channels, settings, seconds, n_windows, w
                                         "msamples_per_s": n_streams * spp / float(np.median(full_wall)) / 1e6}}
     full = pcm.view(n_streams, frames, channels)
     check = rng.choice(n_windows, size=8, replace=False)
+    corpus = ctx.corpus(sea, sea_off, lens, headers)
     for planar in (False, True):
         out = torch.empty(win_samples, dtype=torch.float32 if planar else torch.int16, device=dev)
         torch.cuda.synchronize()
@@ -140,8 +144,57 @@ def shape(ctx, torch, name, n_streams, channels, settings, seconds, n_windows, w
             "call_ms": wall * 1e3, "windows_per_s": n_windows / wall, "window_msamples_per_s": win_samples / wall / 1e6,
             "kernel_ms": float(np.median(kms)), "decode_ms": float(np.median(decs)), "extract_ms": float(np.median(exts)),
             "extract_gbs": win_samples * (2 + (4 if planar else 2)) / (float(np.median(exts)) * 1e-3) / 1e9,
-            "window_calls_per_full_decode": float(np.median(full_wall)) / wall}
+            "window_calls_per_full_decode": float(np.median(full_wall)) / wall,
+            "async": corpus_async(ctx, torch, corpus, ws, ff, W, planar, out, fo, reps)}
+    corpus.close()
+    ctx.set_stream(torch.cuda.current_stream().cuda_stream)
     return row
+
+
+def corpus_async(ctx, torch, corpus, ws, ff, W, planar, ref_out, ref_fo, reps, calls=20):
+    """The registered-corpus form on the same windows: GPU ms per call (CUDA events around `calls` back-to-back calls), host enqueue
+    us per call, graph-replay ms per call (one captured call), and a check that slots and frames_out equal decode_windows_device's."""
+    n = len(ws)
+    si = torch.tensor(ws.astype(np.int64), device="cuda")
+    fi = torch.tensor(ff.astype(np.int64), device="cuda")
+    out = torch.empty_like(ref_out)
+    fo = torch.zeros(n, dtype=torch.int32, device="cuda")
+
+    def call():
+        corpus.decode_windows(si, fi, W, float32_planar=planar, out=out, frames_out=fo)
+
+    call()
+    torch.cuda.synchronize()
+    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    gpu, enq = [], []
+    for _ in range(reps):
+        e0.record()
+        t0 = time.perf_counter()
+        for _ in range(calls):
+            call()
+        enq.append((time.perf_counter() - t0) / calls)
+        e1.record()
+        e1.synchronize()
+        gpu.append(e0.elapsed_time(e1) / calls)
+    equal = bool(torch.equal(out, ref_out)) and bool(np.array_equal(fo.cpu().numpy().astype(np.uint64), ref_fo))
+    side = torch.cuda.Stream()
+    side.wait_stream(torch.cuda.current_stream())
+    g = torch.cuda.CUDAGraph()
+    with torch.cuda.graph(g, stream=side):
+        call()
+    torch.cuda.synchronize()
+    graph = []
+    for _ in range(reps):
+        e0.record()
+        for _ in range(calls):
+            g.replay()
+        e1.record()
+        e1.synchronize()
+        graph.append(e0.elapsed_time(e1) / calls)
+    corpus.check()
+    assert equal, "async slots differ from decode_windows_device's"
+    return {"route": corpus.route, "gpu_ms": float(np.median(gpu)), "enqueue_us": float(np.median(enq)) * 1e6,
+            "graph_replay_ms": float(np.median(graph)), "equal_to_decode_windows_device": equal}
 
 
 def main():
