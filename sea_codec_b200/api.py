@@ -15,6 +15,7 @@ from __future__ import annotations
 
 import ctypes as C
 import os
+import weakref
 from dataclasses import dataclass
 from typing import BinaryIO, List, Optional, Sequence
 
@@ -205,9 +206,12 @@ class Context:
         if rc:
             raise SeaError(rc, "no usable CUDA device for libsea_b200 (there is no CPU fallback)")
         self.device = device
+        self._corpora = weakref.WeakSet()  # sea_b200_corpus_destroy uses its context: they are closed before it
 
     def close(self):
         if getattr(self, "_h", None) and self._h.value:
+            for corpus in list(getattr(self, "_corpora", ())):
+                corpus.close()
             self._L.sea_b200_ctx_destroy(self._h)
             self._h = C.c_void_p()
 
@@ -466,10 +470,15 @@ class Corpus:
         self.route = "fast" if route.value else "generic"
         self.stream_frames_cuda = torch.from_numpy(self.stream_frames.astype(np.int64)).to(self.device)
         self._status = torch.zeros(1, dtype=torch.int32, device=self.device)
+        ctx._corpora.add(self)
 
     def close(self):
         if getattr(self, "_h", None) and self._h.value:
-            self._L.sea_b200_corpus_destroy(self._h)
+            # The garbage collector may finalise a context before a corpus that refers to it (a reference cycle, whose weak
+            # references it clears first): the corpus's device table is then left to the process, not freed through a
+            # destroyed context.
+            if self._ctx._h.value:
+                self._L.sea_b200_corpus_destroy(self._h)
             self._h = C.c_void_p()
 
     def __del__(self):

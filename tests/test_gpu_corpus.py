@@ -12,10 +12,9 @@ import pytest
 
 import sea_codec_b200 as S
 from sea_codec_b200 import api, synth
-from util import ROOT
+from util import ROOT, Packed, run_async, windows
 
 N = 5120
-SENTINEL = -12345
 
 
 # ------------------------------------------------------------------------------------------------ CPU: window plan
@@ -105,30 +104,6 @@ def _encode(ctx, seed, frames, ch, rate=44100, **kw):
     return ctx.sea_encode(synth.gen_stream(seed, frames, ch, rate), rate, ch, S.EncoderSettings(**kw))
 
 
-class Packed:
-    """.sea streams in one device buffer; `shift` moves every stream off 16-byte alignment."""
-
-    def __init__(self, files, shift=0):
-        import torch
-
-        self.files = list(files)
-        offs, t = [], 0
-        for f in self.files:
-            t += shift
-            offs.append(t)
-            t = (t + len(f) + 15) // 16 * 16
-        host = np.zeros(t + 64, dtype=np.uint8)
-        for o, f in zip(offs, self.files):
-            host[o: o + len(f)] = np.frombuffer(f, dtype=np.uint8)
-        self.buf = torch.from_numpy(host).cuda()
-        self.offs = np.array(offs, dtype=np.uint64)
-        self.lens = np.array([len(f) for f in self.files], dtype=np.uint64)
-        self.headers = np.stack([np.frombuffer(f[:22], dtype=np.uint8) for f in self.files])
-
-    def corpus(self, ctx, skip_metadata=False):
-        return ctx.corpus(self.buf, self.offs, self.lens, self.headers, skip_metadata=skip_metadata)
-
-
 def reference(ctx, packed, ch, ws, ff, W, planar, skip_metadata):
     """decode_windows_device's slots (out_offsets = w * W * ch) and frames_out for the same windows."""
     import torch
@@ -139,34 +114,6 @@ def reference(ctx, packed, ch, ws, ff, W, planar, skip_metadata):
     fo = ctx.decode_windows_device(packed.buf.data_ptr(), packed.offs, packed.lens, packed.headers, ws, ff, np.full(n, W), out.data_ptr(),
                                    np.arange(n, dtype=np.uint64) * (W * ch), float32_planar=planar, skip_metadata=skip_metadata)
     return out[: n * W * ch].cpu().numpy(), fo.astype(np.int64)
-
-
-def run_async(corpus, ws, ff, W, planar, pad=5, status=None):
-    """corpus.decode_windows into an odd element offset of a sentinel-filled tensor; checks the sentinels and returns (slots, frames_out)."""
-    import torch
-
-    n, ch = len(ws), corpus.channels
-    total = n * W * ch
-    big = torch.full((total + 2 * pad + 1,), SENTINEL, dtype=torch.float32 if planar else torch.int16, device="cuda")
-    out = big[pad: pad + total]
-    fo = torch.full((max(n, 1),), -7, dtype=torch.int32, device="cuda")[:n]
-    si = torch.tensor(np.asarray(ws, dtype=np.int64), device="cuda")
-    fi = torch.tensor(np.asarray(ff, dtype=np.uint64).astype(np.int64), device="cuda")
-    corpus.decode_windows(si, fi, W, float32_planar=planar, out=out, frames_out=fo, status=status)
-    host = big.cpu().numpy()
-    assert np.all(host[:pad] == SENTINEL) and np.all(host[pad + total:] == SENTINEL), "a byte outside the slots was written"
-    return host[pad: pad + total], fo.cpu().numpy().astype(np.int64)
-
-
-def windows(rng, frames, n, W):
-    """Seeded starts over every stream, with edge starts mixed in: 0, a chunk boundary, the last frame, past the end, near 2^64."""
-    ws = rng.integers(0, len(frames), size=n)
-    ff = np.array([int(rng.integers(0, int(frames[s]) + 100)) for s in ws], dtype=np.uint64)
-    if n:
-        edges = [0, N, N - 1, int(frames[ws[0]]) - 1, int(frames[ws[0]]), 2**64 - 1, 2**64 - N, 2**63]
-        for i, e in enumerate(edges[:n]):
-            ff[i] = e
-    return ws.astype(np.uint32), ff
 
 
 SHAPES = {

@@ -123,8 +123,7 @@ def test_cpp_seaconv_matches_python_cli(ctx, oracle, tmp_path):
     from sea_codec_b200 import build as B
     from util import ROOT
 
-    exe = os.path.join(ROOT, "tests", "build", "seaconv")
-    os.makedirs(os.path.dirname(exe), exist_ok=True)
+    exe = str(tmp_path / "seaconv")  # outside the source tree, which may be read-only
     lib_dir = os.path.dirname(B.LIB)
     subprocess.run(["g++", "-std=c++17", "-O2", "-I" + os.path.join(ROOT, "include"), "-o", exe, os.path.join(ROOT, "tools", "seaconv.cpp"),
                     "-L" + lib_dir, "-l:libsea_b200.so", "-Wl,-rpath," + lib_dir], check=True)

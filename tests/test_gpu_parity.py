@@ -425,9 +425,8 @@ def test_cpp_host_mirror(ctx, oracle, tmp_path):
 
     from sea_codec_b200 import build as B
 
-    exe = os.path.join(ROOT, "tests", "build", "host_mirror_test")
+    exe = str(tmp_path / "host_mirror_test")  # outside the source tree, which may be read-only
     src = os.path.join(ROOT, "tests", "csrc", "host_mirror_test.cpp")
-    os.makedirs(os.path.dirname(exe), exist_ok=True)
     lib_dir = os.path.dirname(B.LIB)
     subprocess.run(["g++", "-std=c++17", "-O2", "-o", exe, src, "-L" + lib_dir, "-l:libsea_b200.so", "-Wl,-rpath," + lib_dir], check=True)
     for channels, bits, vbr in ((2, 3.0, 0), (1, 3.0, 1), (3, 5.0, 0)):

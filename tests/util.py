@@ -8,6 +8,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 REFERENCE_C_GOLDEN = os.path.join(ROOT, "tests", "golden", "reference_c.json")
+SENTINEL = -12345
 
 
 def sha(b) -> str:
@@ -77,3 +78,55 @@ def build_host_math():
     if not os.path.exists(so) or os.path.getmtime(so) < max(os.path.getmtime(src), os.path.getmtime(dep)):
         subprocess.run(["g++", "-O2", "-std=c++17", "-x", "c++", "-shared", "-fPIC", "-fwrapv", "-o", so, src], check=True)
     return so
+
+
+class Packed:
+    """.sea streams in one device buffer; `shift` moves every stream off 16-byte alignment."""
+
+    def __init__(self, files, shift=0):
+        import torch
+
+        self.files = list(files)
+        offs, t = [], 0
+        for f in self.files:
+            t += shift
+            offs.append(t)
+            t = (t + len(f) + 15) // 16 * 16
+        host = np.zeros(t + 64, dtype=np.uint8)
+        for o, f in zip(offs, self.files):
+            host[o: o + len(f)] = np.frombuffer(f, dtype=np.uint8)
+        self.buf = torch.from_numpy(host).cuda()
+        self.offs = np.array(offs, dtype=np.uint64)
+        self.lens = np.array([len(f) for f in self.files], dtype=np.uint64)
+        self.headers = np.stack([np.frombuffer(f[:22], dtype=np.uint8) for f in self.files])
+
+    def corpus(self, ctx, skip_metadata=False):
+        return ctx.corpus(self.buf, self.offs, self.lens, self.headers, skip_metadata=skip_metadata)
+
+
+def windows(rng, frames, n, W, N=5120):
+    """Seeded starts over every stream, with edge starts mixed in: 0, the chunk boundary N, the last frame, past the end, near 2^64."""
+    ws = rng.integers(0, len(frames), size=n)
+    ff = np.array([int(rng.integers(0, int(frames[s]) + 100)) for s in ws], dtype=np.uint64)
+    if n:
+        edges = [0, N, N - 1, int(frames[ws[0]]) - 1, int(frames[ws[0]]), 2**64 - 1, 2**64 - N, 2**63]
+        for i, e in enumerate(edges[:n]):
+            ff[i] = e
+    return ws.astype(np.uint32), ff
+
+
+def run_async(corpus, ws, ff, W, planar, pad=5, status=None):
+    """corpus.decode_windows into an odd element offset of a sentinel-filled tensor; checks the sentinels and returns (slots, frames_out)."""
+    import torch
+
+    n, ch = len(ws), corpus.channels
+    total = n * W * ch
+    big = torch.full((total + 2 * pad + 1,), SENTINEL, dtype=torch.float32 if planar else torch.int16, device="cuda")
+    out = big[pad: pad + total]
+    fo = torch.full((max(n, 1),), -7, dtype=torch.int32, device="cuda")[:n]
+    si = torch.tensor(np.asarray(ws, dtype=np.int64), device="cuda")
+    fi = torch.tensor(np.asarray(ff, dtype=np.uint64).astype(np.int64), device="cuda")
+    corpus.decode_windows(si, fi, W, float32_planar=planar, out=out, frames_out=fo, status=status)
+    host = big.cpu().numpy()
+    assert np.all(host[:pad] == SENTINEL) and np.all(host[pad + total:] == SENTINEL), "a byte outside the slots was written"
+    return host[pad: pad + total], fo.cpu().numpy().astype(np.int64)
