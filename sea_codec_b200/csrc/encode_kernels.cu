@@ -12,6 +12,7 @@
 // reference loop would have kept (trap T1), and the winner's state is written back before the next block.
 // The serialized chunk is assembled in shared memory as a big-endian bit string and written out per chunk.
 #include <stdlib.h>
+#include <string.h>
 
 #include "sea_kernels.h"
 
@@ -1075,6 +1076,14 @@ cudaError_t launch_encode_generic(const int16_t *d_pcm, uint8_t *d_out, const En
             else if (other + e * 128u <= budget) lut_mode = kEncLut32;
             else if (p.s == 4u && other + e * 64u <= budget) lut_mode = kEncLut16;
             else lut_mode = kEncLutGlobal;
+            // SEA_B200_ENC_LUT=32|16|global pins the VBR layout whatever the batch size (tests, tuning); a layout that does not
+            // apply (16 needs scale_factor_bits 4) or would take the CTA past 200 KB leaves the choice above
+            const char *pin = p.vbr ? getenv("SEA_B200_ENC_LUT") : nullptr;
+            if (pin) {
+                const int want = !strcmp(pin, "32") ? kEncLut32 : !strcmp(pin, "16") ? kEncLut16 : !strcmp(pin, "global") ? kEncLutGlobal : -1;
+                const size_t need = want == kEncLut32 ? e * 128u : (want == kEncLut16 ? e * 64u : 0u);
+                if (want >= 0 && (want != kEncLut16 || p.s == 4u) && other + need <= 200u * 1024u) lut_mode = want;
+            }
             if (lut_mode != kEncLutGlobal) smem += e * (lut_mode == kEncLut32 ? 128u : 64u);
         }
         smem += 4u * nsf * 4u;  // reciprocals [slot][2^s]
