@@ -390,6 +390,7 @@ struct EncodeJob {
     EncodePlan plan;
     EncParams params;
     std::vector<EncStream> streams;
+    uint32_t chunk_buf_bytes;  // the largest chunk these streams can produce (launch_encode_generic)
 };
 
 int plan_encode(sea_b200_ctx *ctx, uint32_t n_streams, const uint64_t *pcm_offsets, const uint32_t *n_frames, uint32_t sample_rate,
@@ -417,6 +418,10 @@ int plan_encode(sea_b200_ctx *ctx, uint32_t n_streams, const uint64_t *pcm_offse
     p.n_streams = n_streams;
     job->streams.resize(n_streams);
     bool any_full = false;
+    // CBR: every chunk of a job fits max_chunk_bytes exactly.  VBR: a full chunk is full_chunk_bytes exactly; a last chunk of `last`
+    // frames is bounded by its own bucket counts with every block taken at F frames (the items past `sortable` keep size `base`)
+    // and by `last` frames at base+2 bits.
+    job->chunk_buf_bytes = pl.vbr ? 0u : pl.max_chunk_bytes;
     for (uint32_t i = 0; i < n_streams; i++) {
         EncStream &e = job->streams[i];
         memset(&e, 0, sizeof(e));
@@ -434,8 +439,15 @@ int plan_encode(sea_b200_ctx *ctx, uint32_t n_streams, const uint64_t *pcm_offse
             e.last_counts[2] = (uint32_t)counts[3];
             if ((counts[0] && pl.base < 2) || (counts[2] && pl.base + 1 > 8) || (counts[3] && pl.base + 2 > 8))
                 return fail(ctx, SEA_B200_ERR_DOMAIN, "VBR bitrate produces a residual size outside 1..8 (common.rs:34 panics)");
+            const uint64_t items = ((uint64_t)last + pl.F - 1) / pl.F * channels;
+            const uint64_t size_sum = counts[0] * (pl.base - 1) + (counts[1] + items - sortable) * pl.base + counts[2] * (pl.base + 1) +
+                                      counts[3] * (pl.base + 2);
+            const uint64_t bits = std::min<uint64_t>(size_sum * pl.F, (uint64_t)last * channels * (pl.base + 2));
+            const uint64_t bytes = 4 + 16ull * channels + (items * pl.s + 7) / 8 + (items * 2 + 7) / 8 + (bits + 7) / 8;
+            job->chunk_buf_bytes = std::max<uint32_t>(job->chunk_buf_bytes, (uint32_t)std::min<uint64_t>(bytes, pl.max_chunk_bytes));
         }
     }
+    if (pl.vbr && any_full) job->chunk_buf_bytes = std::max(job->chunk_buf_bytes, pl.full_chunk_bytes);
     if (any_full && !pl.full_chunk_valid)
         return fail(ctx, SEA_B200_ERR_DOMAIN, "VBR bitrate produces a residual size outside 1..8 (common.rs:34 panics)");
     return SEA_B200_OK;
@@ -458,7 +470,8 @@ int enqueue_encode(sea_b200_ctx *ctx, EncodeJob &job, const int16_t *d_pcm, uint
     if (!descriptors_uploaded)
         CU(cudaMemcpyAsync(d_streams, job.streams.data(), sizeof(EncStream) * n, cudaMemcpyHostToDevice, ctx->stream));
     CU(launch_encode_generic(d_pcm, d_out, d_streams, job.params, ctx->tabs, d_state, ctx->lens.as<uint64_t>() + (size_t)slot * n,
-                             ctx->chunk0.as<uint32_t>() + (size_t)slot * n, ctx->ties.as<unsigned long long>(), ws, ctx->d_err, ctx->stream));
+                             ctx->chunk0.as<uint32_t>() + (size_t)slot * n, ctx->ties.as<unsigned long long>(), ws, ctx->d_err, ctx->stream,
+                             job.chunk_buf_bytes));
     ctx->launches++;
     return SEA_B200_OK;
 }
@@ -484,7 +497,7 @@ int run_encode(sea_b200_ctx *ctx, EncodeJob &job, const int16_t *d_pcm, uint8_t 
     ctx->h_ties.assign((size_t)n + 1u, 0ull);
     CU(cudaEventRecord(ctx->ev0, ctx->stream));
     CU(launch_encode_generic(d_pcm, d_out, ctx->streams.as<EncStream>(), job.params, ctx->tabs, d_state, ctx->lens.as<uint64_t>(),
-                             ctx->chunk0.as<uint32_t>(), ctx->ties.as<unsigned long long>(), ws, ctx->d_err, ctx->stream));
+                             ctx->chunk0.as<uint32_t>(), ctx->ties.as<unsigned long long>(), ws, ctx->d_err, ctx->stream, job.chunk_buf_bytes));
     ctx->launches++;
     CU(cudaEventRecord(ctx->ev1, ctx->stream));
     int dev_err = 0;

@@ -60,6 +60,7 @@ cudaError_t launch_corpus_validate(const uint8_t *d_sea, const CorpusStream *d_s
 {
     if (total_chunks == 0) return cudaSuccess;
     const uint64_t blocks = (total_chunks + 127) / 128;
+    debug_launch("corpus_validate: %u channels, %llu CTAs", channels, (unsigned long long)blocks);
     corpus_validate_kernel<<<(unsigned)blocks, 128, 0, stream>>>(d_sea, d_streams, n_streams, total_chunks, channels, ref_word,
                                                                  d_first_bad, d_mixed);
     return cudaGetLastError();
@@ -410,6 +411,7 @@ static cudaError_t launch_corpus_fast(const CorpusLaunch &p, const int32_t *tab,
     using Cfg = CorpusCfg<C, BT>;
     const uint64_t per_cta = (uint64_t)kCorpusWarps * Cfg::kRows, blocks = (units + per_cta - 1) / per_cta;
     const size_t smem = Cfg::smem(p.s);
+    debug_launch("corpus_fast<%d,%d,%d>: %zu B smem, %llu CTAs", C, BT, (int)p.planar, smem, (unsigned long long)blocks);
     if (p.planar) corpus_fast_kernel<C, BT, true><<<(unsigned)blocks, kCorpusWarps * 32, smem, stream>>>(p, tab, units);
     else corpus_fast_kernel<C, BT, false><<<(unsigned)blocks, kCorpusWarps * 32, smem, stream>>>(p, tab, units);
     return cudaGetLastError();
@@ -421,6 +423,7 @@ cudaError_t launch_corpus_windows(const CorpusLaunch &p, bool fast, DevTables ta
     if (units == 0) return cudaSuccess;
     if (!fast) {
         const uint64_t chains = units * p.channels, blocks = (chains + 127) / 128;
+        debug_launch("corpus_generic: %u channels, planar %d, %llu CTAs", p.channels, (int)p.planar, (unsigned long long)blocks);
         corpus_generic_kernel<<<(unsigned)blocks, 128, 0, stream>>>(p, tabs, chains);
         return cudaGetLastError();
     }

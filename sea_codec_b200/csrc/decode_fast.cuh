@@ -391,7 +391,7 @@ static cudaError_t launch_unrolled_p(const uint8_t *d_sea, int16_t *d_pcm, const
     if (e != cudaSuccess) return e;
     // The carve-out is left to the driver (the smallest that holds the resident CTAs): the kernel wants its L1 -- pinned to the
     // maximum shared-memory carve-out the config-4 launch takes 17.4 instead of 13.9 ms (profiles/r02_s2_probe_pairfetch.txt).
-    if (getenv("SEA_B200_DEBUG_LAUNCH")) fprintf(stderr, "decode_unrolled<%d,%d,%d,%d,%d>: %u warps/CTA, %zu B smem, %llu CTAs\n", C, B, kMode, S, (int)PAIR, warps, smem, (unsigned long long)blocks);
+    debug_launch("decode_unrolled<%d,%d,%d,%d,%d>: %u warps/CTA, %zu B smem, %llu CTAs", C, B, kMode, S, (int)PAIR, warps, smem, (unsigned long long)blocks);
     decode_unrolled_kernel<C, B, kMode, S, PAIR><<<(unsigned)blocks, warps * 32, smem, stream>>>(d_sea, d_pcm, d_streams, p, tab, d_err);
     return cudaGetLastError();
 }

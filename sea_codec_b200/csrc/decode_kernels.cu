@@ -65,6 +65,7 @@ cudaError_t launch_decode_generic(const uint8_t *d_sea, int16_t *d_pcm, const De
     if (total_chains == 0) return cudaSuccess;
     const uint32_t threads = 128;
     const uint64_t blocks = (total_chains + threads - 1) / threads;
+    debug_launch("decode_generic: %u threads/CTA, %llu CTAs, %llu chains", threads, (unsigned long long)blocks, (unsigned long long)total_chains);
     decode_generic_kernel<<<(unsigned)blocks, threads, 0, stream>>>(d_sea, d_pcm, d_streams, n_streams, total_chains, tabs, d_err);
     return cudaGetLastError();
 }
@@ -319,6 +320,7 @@ static cudaError_t launch_staged(const uint8_t *d_sea, uint64_t sea_len, int16_t
     if (e != cudaSuccess) return e;
     const uint64_t chunks_per_cta = (uint64_t)kWarpsPerCta * Cfg::kRows;
     const uint64_t blocks = (p.total_chunks + chunks_per_cta - 1) / chunks_per_cta;
+    debug_launch("decode_staged<%d,%d>: %u warps/CTA, %zu B smem, %llu CTAs", C, BT, (unsigned)kWarpsPerCta, smem, (unsigned long long)blocks);
     decode_staged_kernel<C, BT><<<(unsigned)blocks, kWarpsPerCta * 32, smem, stream>>>(d_sea, sea_len, d_pcm, d_streams, p, tab, d_err);
     return cudaGetLastError();
 }

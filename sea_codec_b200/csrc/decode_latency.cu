@@ -317,6 +317,7 @@ cudaError_t launch_decode_latency(const uint8_t *d_sea, int16_t *d_pcm, const De
         if (e != cudaSuccess) return e;
         if (dev >= 0 && dev < 64) configured[dev] = true;
     }
+    debug_launch("decode_latency: %u channels, %u warps/CTA, %zu B smem, %llu CTAs", channels, kLatWarps, smem, (unsigned long long)total_chunks);
     decode_latency_kernel<<<(unsigned)total_chunks, kLatThreads, smem, stream>>>(d_sea, d_pcm, d_streams, n_streams, total_chunks, chunk_size, tabs,
                                                                         d_err);
     return cudaGetLastError();

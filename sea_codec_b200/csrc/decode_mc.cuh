@@ -324,6 +324,7 @@ static cudaError_t launch_mc(const uint8_t *d_sea, int16_t *d_pcm, const DecStre
     if (e != cudaSuccess) return e;
     const uint64_t chunks_per_cta = (uint64_t)warps * Cfg::kChunksPerWarp;
     const uint64_t blocks = (p.total_chunks + chunks_per_cta - 1) / chunks_per_cta;
+    debug_launch("decode_mc<%d,%d,%d>: %u warps/CTA, %zu B smem, %llu CTAs", CT, B, (int)S4, warps, smem, (unsigned long long)blocks);
     decode_mc_kernel<CT, B, S4><<<(unsigned)blocks, warps * 32, smem, stream>>>(d_sea, d_pcm, d_streams, p, tab, d_err);
     return cudaGetLastError();
 }

@@ -348,6 +348,7 @@ static cudaError_t launch_vbr(const uint8_t *d_sea, int16_t *d_pcm, const DecStr
     if (e != cudaSuccess) return e;
     const uint64_t chunks_per_cta = (uint64_t)Cfg::kWarps * Cfg::kRows;
     const uint64_t blocks = (p.total_chunks + chunks_per_cta - 1) / chunks_per_cta;
+    debug_launch("decode_vbr<%d,%d,%d,%d>: %u warps/CTA, %zu B smem, %llu CTAs", C, RS, (int)S4, KF, (unsigned)Cfg::kWarps, smem, (unsigned long long)blocks);
     decode_vbr_kernel<C, RS, S4, KF><<<(unsigned)blocks, Cfg::kWarps * 32, smem, stream>>>(d_sea, d_pcm, d_streams, p, tab, d_err);
     return cudaGetLastError();
 }

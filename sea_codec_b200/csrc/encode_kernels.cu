@@ -1038,13 +1038,14 @@ static cudaError_t launch_encode_t(const int16_t *d_pcm, uint8_t *d_out, const E
     // 164 KB of the 228 KB and left a second wave at the high bitrates)
     e = cudaFuncSetAttribute(encode_kernel<FB, S>, cudaFuncAttributePreferredSharedMemoryCarveout, (int)cudaSharedmemCarveoutMaxShared);
     if (e != cudaSuccess) return e;
+    debug_launch("encode_kernel<%d,%d>: %u channels, %u threads/CTA, %zu B smem, %u CTAs", FB, S, p.channels, T, smem, p.n_streams);
     encode_kernel<FB, S><<<p.n_streams, T, smem, stream>>>(d_pcm, d_out, d_streams, p, tabs, d_state, d_out_lens, d_chunk0, d_ties, ws, d_err);
     return cudaGetLastError();
 }
 
 cudaError_t launch_encode_generic(const int16_t *d_pcm, uint8_t *d_out, const EncStream *d_streams, const EncParams &p,
                                   DevTables tabs, int32_t *d_state, uint64_t *d_out_lens, uint32_t *d_chunk0,
-                                  unsigned long long *d_ties, EncWorkspace ws, int *d_err, cudaStream_t stream)
+                                  unsigned long long *d_ties, EncWorkspace ws, int *d_err, cudaStream_t stream, uint32_t chunk_buf_bytes)
 {
     if (p.n_streams == 0) return cudaSuccess;
     const uint32_t nsf = 1u << p.s, lpc = nsf < 32u ? nsf : 32u, cpw = 32u / lpc;
@@ -1059,48 +1060,68 @@ cudaError_t launch_encode_generic(const int16_t *d_pcm, uint8_t *d_out, const En
     if (const char *env = getenv("SEA_B200_ENC_SPLIT")) split = fast && p.channels >= 2u && env[0] == '1';
     uint32_t warps = split ? p.channels : (p.channels + cpw - 1u) / cpw;
     if (warps > 8u) warps = 8u;
-    const uint32_t T = warps * 32u;
-    size_t smem = ((size_t)(p.max_chunk_bytes + 3u) / 4u + 2u) * 4u + (size_t)p.channels * 17u * 4u + ((2u * (size_t)p.F * T + 15u) & ~(size_t)15u) + 16u;
-    int lut_mode = kEncLut32;
-    if (fast) {
-        smem += ((size_t)warps * cpw * p.F * 2u + 15u) & ~(size_t)15u;
-        {   // One CTA per stream, all of them resident at once if they fit: with k = ceil(streams / 148) CTAs per SM a CTA may use
-            // 227 KB / k less the 1 KB the hardware reserves per CTA (31 KB at the benchmark's 1024 streams); with more streams
-            // than that would leave 28 KB for, keep the CTA at or under 28 KB (8 per SM, several waves).
-            const int fb = p.vbr ? 0 : (int)p.hdr_bits;
-            const size_t e = enc_lut_entries(fb, p.base), other = smem + 256u + (p.vbr ? (size_t)enc_vbr_scratch_bytes(p) + 16u : 0u);
-            const size_t per_sm = (p.n_streams + 147u) / 148u;
-            size_t budget = 227u * 1024u / per_sm;
-            budget = budget > 1280u + 28u * 1024u ? budget - 1280u : 28u * 1024u;
-            if (!p.vbr) lut_mode = enc_lut_mode_cbr(fb, (int)p.s);
-            else if (other + e * 128u <= budget) lut_mode = kEncLut32;
-            else if (p.s == 4u && other + e * 64u <= budget) lut_mode = kEncLut16;
-            else lut_mode = kEncLutGlobal;
-            // SEA_B200_ENC_LUT=32|16|global pins the VBR layout whatever the batch size (tests, tuning); a layout that does not
-            // apply (16 needs scale_factor_bits 4) or would take the CTA past 200 KB leaves the choice above
-            const char *pin = p.vbr ? getenv("SEA_B200_ENC_LUT") : nullptr;
-            if (pin) {
-                const int want = !strcmp(pin, "32") ? kEncLut32 : !strcmp(pin, "16") ? kEncLut16 : !strcmp(pin, "global") ? kEncLutGlobal : -1;
-                const size_t need = want == kEncLut32 ? e * 128u : (want == kEncLut16 ? e * 64u : 0u);
-                if (want >= 0 && (want != kEncLut16 || p.s == 4u) && other + need <= 200u * 1024u) lut_mode = want;
+    // The CTA's shared memory for a chunk buffer of chunk_bytes and `warps` warps; also picks the VBR table layout (fast pass) and
+    // the offset of the VBR scratch when it is kept in shared memory (0: global workspace).
+    auto layout = [&](uint32_t chunk_bytes, uint32_t warps, int &lut_mode, uint32_t &vbr_smem_off) -> size_t {
+        const uint32_t T = warps * 32u;
+        size_t smem = ((size_t)(chunk_bytes + 3u) / 4u + 2u) * 4u + (size_t)p.channels * 17u * 4u + ((2u * (size_t)p.F * T + 15u) & ~(size_t)15u) + 16u;
+        lut_mode = kEncLut32;
+        if (fast) {
+            smem += ((size_t)warps * cpw * p.F * 2u + 15u) & ~(size_t)15u;
+            {   // One CTA per stream, all of them resident at once if they fit: with k = ceil(streams / 148) CTAs per SM a CTA may use
+                // 227 KB / k less the 1 KB the hardware reserves per CTA (31 KB at the benchmark's 1024 streams); with more streams
+                // than that would leave 28 KB for, keep the CTA at or under 28 KB (8 per SM, several waves).
+                const int fb = p.vbr ? 0 : (int)p.hdr_bits;
+                const size_t e = enc_lut_entries(fb, p.base), other = smem + 256u + (p.vbr ? (size_t)enc_vbr_scratch_bytes(p) + 16u : 0u);
+                const size_t per_sm = (p.n_streams + 147u) / 148u;
+                size_t budget = 227u * 1024u / per_sm;
+                budget = budget > 1280u + 28u * 1024u ? budget - 1280u : 28u * 1024u;
+                if (!p.vbr) lut_mode = enc_lut_mode_cbr(fb, (int)p.s);
+                else if (other + e * 128u <= budget) lut_mode = kEncLut32;
+                else if (p.s == 4u && other + e * 64u <= budget) lut_mode = kEncLut16;
+                else lut_mode = kEncLutGlobal;
+                // SEA_B200_ENC_LUT=32|16|global pins the VBR layout whatever the batch size (tests, tuning); a layout that does not
+                // apply (16 needs scale_factor_bits 4) or would take the CTA past 200 KB leaves the choice above
+                const char *pin = p.vbr ? getenv("SEA_B200_ENC_LUT") : nullptr;
+                if (pin) {
+                    const int want = !strcmp(pin, "32") ? kEncLut32 : !strcmp(pin, "16") ? kEncLut16 : !strcmp(pin, "global") ? kEncLutGlobal : -1;
+                    const size_t need = want == kEncLut32 ? e * 128u : (want == kEncLut16 ? e * 64u : 0u);
+                    if (want >= 0 && (want != kEncLut16 || p.s == 4u) && other + need <= 200u * 1024u) lut_mode = want;
+                }
+                if (lut_mode != kEncLutGlobal) smem += e * (lut_mode == kEncLut32 ? 128u : 64u);
             }
-            if (lut_mode != kEncLutGlobal) smem += e * (lut_mode == kEncLut32 ? 128u : 64u);
+            smem += 4u * nsf * 4u;  // reciprocals [slot][2^s]
         }
-        smem += 4u * nsf * 4u;  // reciprocals [slot][2^s]
+        vbr_smem_off = 0;
+        if (p.vbr) {  // keep the per-chunk VBR scratch in shared memory when it is small (stereo: 8.7 KB)
+            const uint64_t sc = enc_vbr_scratch_bytes(p);
+            if (sc <= 40u * 1024u && smem + sc + 16u <= 200u * 1024u) {
+                smem = (smem + 15u) & ~(size_t)15u;
+                vbr_smem_off = (uint32_t)smem;
+                smem += sc;
+            }
+        }
+        return smem;
+    };
+    uint32_t chunk_bytes = p.max_chunk_bytes, vbr_smem_off = 0;
+    int lut_mode = kEncLut32;
+    size_t smem = layout(chunk_bytes, warps, lut_mode, vbr_smem_off);
+    // Some settings make_encode_plan accepts do not fit 200 KB under that sizing: VBR chunks near 64 KB, whose max_chunk_bytes (every
+    // sample at base+2 bits) is up to ~3x the largest chunk the job can produce, and 160 or more channels with long blocks, whose
+    // code double buffer takes 2 F x 256 bytes at 8 warps.  Those (and only those) size the chunk buffer from the job's largest
+    // chunk, then give the generic pass fewer warps (its chain groups loop over any warp count).
+    if (smem > 200u * 1024u && chunk_buf_bytes < chunk_bytes) {
+        chunk_bytes = chunk_buf_bytes;
+        smem = layout(chunk_bytes, warps, lut_mode, vbr_smem_off);
     }
+    while (smem > 200u * 1024u && !fast && warps > 1u) smem = layout(chunk_bytes, --warps, lut_mode, vbr_smem_off);
+    if (smem > 200u * 1024u) return cudaErrorInvalidConfiguration;
+    const uint32_t T = warps * 32u;
     EncParams pp = p;
-    pp.vbr_smem_off = 0;
+    pp.max_chunk_bytes = chunk_bytes;
+    pp.vbr_smem_off = vbr_smem_off;
     pp.lut_mode = (uint32_t)lut_mode;
     pp.split = split ? 1u : 0u;
-    if (p.vbr) {  // keep the per-chunk VBR scratch in shared memory when it is small (stereo: 8.7 KB)
-        const uint64_t sc = enc_vbr_scratch_bytes(p);
-        if (sc <= 40u * 1024u && smem + sc + 16u <= 200u * 1024u) {
-            smem = (smem + 15u) & ~(size_t)15u;
-            pp.vbr_smem_off = (uint32_t)smem;
-            smem += sc;
-        }
-    }
-    if (smem > 200u * 1024u) return cudaErrorInvalidConfiguration;
 #define SEA_ENC(FBV, SV) return launch_encode_t<FBV, SV>(d_pcm, d_out, d_streams, pp, tabs, d_state, d_out_lens, d_chunk0, d_ties, ws, d_err, stream, T, smem)
 #define SEA_ENC_S(SV)                      \
     {                                      \

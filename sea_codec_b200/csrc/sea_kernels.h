@@ -1,12 +1,27 @@
 // sea_kernels.h -- launch interface between the C-ABI layer (capi.cu) and the CUDA kernels.
 #pragma once
 #include <cuda_runtime.h>
+#include <stdarg.h>
 #include <stdint.h>
+#include <stdio.h>
 #include <stdlib.h>
 
 #include "sea_common.cuh"
 
 namespace sea {
+
+// SEA_B200_DEBUG_LAUNCH set: every decode and encode launch prints one line to stderr, "<kernel>: <shape>", before it is queued
+// (tests read it to see which route ran).  Unset: nothing is printed.
+inline void debug_launch(const char *fmt, ...) __attribute__((format(printf, 1, 2)));
+inline void debug_launch(const char *fmt, ...)
+{
+    if (!getenv("SEA_B200_DEBUG_LAUNCH")) return;
+    va_list ap;
+    va_start(ap, fmt);
+    vfprintf(stderr, fmt, ap);
+    va_end(ap);
+    fputc('\n', stderr);
+}
 
 // Device-side error codes written to the error word by kernels (first failure wins).
 enum : int { kDevOk = 0, kDevInvalidFrame = 1, kDevDomain = 2, kDevFallback = 3 /* staged kernel: use the generic path */ };
@@ -177,9 +192,11 @@ uint64_t enc_vbr_scratch_bytes(const EncParams &p);
 
 // d_state: nullable; when set, n_streams * channels * 9 int32 loaded at start and stored at the end.
 // d_out_lens: per stream total bytes written; d_chunk0: per stream size of its first chunk; d_ties: VBR boundary ties.
+// chunk_buf_bytes: the largest chunk the launch's streams can produce (<= p.max_chunk_bytes); sizes the chunk buffer only when the
+// CTA would not fit 200 KB with p.max_chunk_bytes.
 cudaError_t launch_encode_generic(const int16_t *d_pcm, uint8_t *d_out, const EncStream *d_streams, const EncParams &p,
                                   DevTables tabs, int32_t *d_state, uint64_t *d_out_lens, uint32_t *d_chunk0,
-                                  unsigned long long *d_ties, EncWorkspace ws, int *d_err, cudaStream_t stream);
+                                  unsigned long long *d_ties, EncWorkspace ws, int *d_err, cudaStream_t stream, uint32_t chunk_buf_bytes);
 
 // ---- measurement -------------------------------------------------------------------------------------------
 cudaError_t launch_int32_peak(int mode, uint32_t *d_sink, uint64_t *lane_ops, cudaStream_t stream);

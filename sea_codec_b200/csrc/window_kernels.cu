@@ -139,6 +139,7 @@ cudaError_t launch_window_extract(const int16_t *d_scratch, void *d_out, const W
     if (n_windows == 0 || max_slot_samples == 0) return cudaSuccess;
     const uint64_t bx = (max_slot_samples + kWinSlotSamplesPerCta - 1u) / kWinSlotSamplesPerCta;
     const dim3 grid((unsigned)(bx < (1u << 20) ? bx : (1u << 20)), n_windows < 65535u ? n_windows : 65535u);
+    debug_launch("window_extract<%d>: %u x %u CTAs", (int)planar_f32, grid.x, grid.y);
     if (planar_f32) window_extract_kernel<true><<<grid, kWinThreads, 0, stream>>>(d_scratch, d_out, d_desc, n_windows);
     else window_extract_kernel<false><<<grid, kWinThreads, 0, stream>>>(d_scratch, d_out, d_desc, n_windows);
     return cudaGetLastError();
