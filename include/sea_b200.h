@@ -201,6 +201,45 @@ int sea_b200_encoder_make_chunks(sea_b200_encoder *enc, const int16_t *pcm, uint
 int sea_b200_decoder_decode_chunks(sea_b200_decoder *dec, sea_b200_ctx *ctx, const uint8_t *chunks, uint64_t len,
                                    int64_t remaining_frames, int16_t *pcm, uint64_t pcm_cap_samples, uint64_t *n_samples);
 
+/* ---------------------------------------------------------------- session pool (many live streams, one launch per push) */
+
+/* A slot table of up to max_sessions streaming encoders with one channel count, sample rate and settings (settings are checked
+ * as sea_b200_encoder_create checks them).  Each open session is the encoder of one live stream: its LMS state and
+ * prev_scalefactor (encoder_base.rs:181-182) and the fewer than frames_per_chunk frames it has buffered stay on the device
+ * between calls.  A push takes a packet of any length from each of its sessions and encodes every chunk that has completed,
+ * across all of them, in one launch.  A pool uses ctx's current stream, is used from one host thread, and must be destroyed
+ * before ctx. */
+typedef struct sea_b200_encoder_pool sea_b200_encoder_pool;
+int sea_b200_encoder_pool_create(sea_b200_ctx *ctx, uint32_t max_sessions, uint32_t channels, uint32_t sample_rate,
+                                 const sea_b200_settings *settings, sea_b200_encoder_pool **pool);
+void sea_b200_encoder_pool_destroy(sea_b200_encoder_pool *pool); /* waits for the context's stream */
+/* Opens slots sessions[0..n) (each < max_sessions, not open, listed once): each starts from EncoderBase::new state with nothing
+ * buffered.  Host-side only. */
+int sea_b200_encoder_pool_open(sea_b200_encoder_pool *pool, uint32_t n, const uint32_t *sessions);
+/* Frames buffered per session (< frames_per_chunk; 0 for a closed slot). */
+int sea_b200_encoder_pool_buffered(const sea_b200_encoder_pool *pool, uint32_t n, const uint32_t *sessions, uint32_t *frames);
+/* Bytes a push of n_frames to an open session produces: k * full chunk bytes for the k chunks it completes, and with `end` the
+ * bound of its short final chunk on top (exact for CBR). */
+int sea_b200_encoder_pool_push_bound(const sea_b200_encoder_pool *pool, uint32_t session, uint64_t n_frames, bool end, uint64_t *bytes);
+/* Appends n_frames[i] interleaved frames at pcm + pcm_offsets[i] (samples) to session sessions[i] and writes every chunk now
+ * complete, back to back, at out + out_offsets[i] (bytes): out_lens[i] = their byte count, n_chunks[i] (nullable) = their
+ * number.  end[i] != 0 (end nullable = none) also encodes what is left as the session's short final chunk and closes the slot.
+ * Joining a session's outputs gives exactly the chunks sea_b200_encode writes after its 22-byte header for the session's whole
+ * PCM, whatever the packet boundaries and whichever sessions share a call; the header is the caller's, with chunk_size = the
+ * session's first chunk's size (file.rs:166-168).  Refused before anything is enqueued, with every session left as it was: a
+ * session not open, >= max_sessions or listed twice, a NULL pointer, buffered plus pushed frames past 2^32
+ * (SEA_B200_ERR_TOO_MANY_FRAMES), an out_caps[i] (nullable = trust the caller) below push_bound (SEA_B200_ERR_CAPACITY).  A
+ * device error closes the call's sessions.  sea_b200_last_vbr_ties_per_stream then holds the call's sessions in call order.
+ * Host buffers (pinned recommended); one launch each for ingest, encode (skipped when no chunk completes) and commit. */
+int sea_b200_encoder_pool_push(sea_b200_encoder_pool *pool, uint32_t n, const uint32_t *sessions, const int16_t *pcm,
+                               const uint64_t *pcm_offsets, const uint32_t *n_frames, const uint8_t *end, uint8_t *out,
+                               const uint64_t *out_offsets, const uint64_t *out_caps, uint64_t *out_lens, uint32_t *n_chunks);
+/* The same with d_pcm and d_out in device memory of ctx's GPU (offsets and lengths stay on the host); bytes of d_out outside
+ * [out_offsets[i], out_offsets[i] + out_lens[i]) are never written. */
+int sea_b200_encoder_pool_push_device(sea_b200_encoder_pool *pool, uint32_t n, const uint32_t *sessions, const int16_t *d_pcm,
+                                      const uint64_t *pcm_offsets, const uint32_t *n_frames, const uint8_t *end, uint8_t *d_out,
+                                      const uint64_t *out_offsets, const uint64_t *out_caps, uint64_t *out_lens, uint32_t *n_chunks);
+
 /* ---------------------------------------------------------------- random access (README.md:125 "seeking" future work) */
 
 /* Decodes frames [first_frame, first_frame + n_frames) of a complete .sea file: only the chunks that cover the range are

@@ -108,6 +108,52 @@ private:
     std::vector<uint64_t> stream_frames_;
 };
 
+// A pool of streaming encoder sessions (sea_b200_encoder_pool_*): one push per round of packets encodes every chunk that completed
+// across all sessions in one launch.  Destroy it before its Context.
+class EncoderPool {
+public:
+    EncoderPool(Context &ctx, uint32_t channels, uint32_t sample_rate, const EncoderSettings &settings, uint32_t max_sessions)
+        : ctx_(&ctx)
+    {
+        sea_b200_settings s = settings.c();
+        ctx.check(sea_b200_encoder_pool_create(ctx.get(), max_sessions, channels, sample_rate, &s, &pool_));
+    }
+    ~EncoderPool() { sea_b200_encoder_pool_destroy(pool_); }
+    EncoderPool(const EncoderPool &) = delete;
+    EncoderPool &operator=(const EncoderPool &) = delete;
+    sea_b200_encoder_pool *get() const { return pool_; }
+    void open(uint32_t n, const uint32_t *sessions) { ctx_->check(sea_b200_encoder_pool_open(pool_, n, sessions)); }
+    void buffered(uint32_t n, const uint32_t *sessions, uint32_t *frames) const
+    {
+        ctx_->check(sea_b200_encoder_pool_buffered(pool_, n, sessions, frames));
+    }
+    uint64_t push_bound(uint32_t session, uint64_t n_frames, bool end) const
+    {
+        uint64_t b = 0;
+        ctx_->check(sea_b200_encoder_pool_push_bound(pool_, session, n_frames, end, &b));
+        return b;
+    }
+    // host buffers; arguments as sea_b200_encoder_pool_push
+    void push(uint32_t n, const uint32_t *sessions, const int16_t *pcm, const uint64_t *pcm_offsets, const uint32_t *n_frames,
+              const uint8_t *end, uint8_t *out, const uint64_t *out_offsets, const uint64_t *out_caps, uint64_t *out_lens,
+              uint32_t *n_chunks = nullptr)
+    {
+        ctx_->check(sea_b200_encoder_pool_push(pool_, n, sessions, pcm, pcm_offsets, n_frames, end, out, out_offsets, out_caps, out_lens, n_chunks));
+    }
+    // device buffers of the context's GPU; arguments as sea_b200_encoder_pool_push_device
+    void push_device(uint32_t n, const uint32_t *sessions, const int16_t *d_pcm, const uint64_t *pcm_offsets, const uint32_t *n_frames,
+                     const uint8_t *end, uint8_t *d_out, const uint64_t *out_offsets, const uint64_t *out_caps, uint64_t *out_lens,
+                     uint32_t *n_chunks = nullptr)
+    {
+        ctx_->check(sea_b200_encoder_pool_push_device(pool_, n, sessions, d_pcm, pcm_offsets, n_frames, end, d_out, out_offsets, out_caps,
+                                                      out_lens, n_chunks));
+    }
+
+private:
+    Context *ctx_;
+    sea_b200_encoder_pool *pool_ = nullptr;
+};
+
 // Every GPU of the box behind one handle (sea_b200_multi, SURVEY 8e): batch calls shard the streams over the GPUs in-process --
 // one context and one host thread per GPU, nothing exchanged between them -- and report per-GPU counts.
 class MultiContext {

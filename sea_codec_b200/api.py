@@ -165,6 +165,15 @@ SYMBOLS = {
     "sea_b200_multi_decode_batch": (C.c_int, [C.c_void_p, C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                               C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "sea_b200_last_vbr_ties_per_stream": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint32]),
+    "sea_b200_encoder_pool_create": (C.c_int, [C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32, C.POINTER(_Settings), C.POINTER(C.c_void_p)]),
+    "sea_b200_encoder_pool_destroy": (None, [C.c_void_p]),
+    "sea_b200_encoder_pool_open": (C.c_int, [C.c_void_p, C.c_uint32, C.c_void_p]),
+    "sea_b200_encoder_pool_buffered": (C.c_int, [C.c_void_p, C.c_uint32, C.c_void_p, C.c_void_p]),
+    "sea_b200_encoder_pool_push_bound": (C.c_int, [C.c_void_p, C.c_uint32, C.c_uint64, C.c_bool, _u64p]),
+    "sea_b200_encoder_pool_push": (C.c_int, [C.c_void_p, C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                             C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "sea_b200_encoder_pool_push_device": (C.c_int, [C.c_void_p, C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                                    C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "sea_b200_synth_pcm_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint32, C.c_uint32, C.c_uint32, C.c_void_p, C.c_void_p,
                                             C.c_void_p, C.c_uint64, C.c_int32, C.c_int32]),
 }
@@ -207,11 +216,14 @@ class Context:
             raise SeaError(rc, "no usable CUDA device for libsea_b200 (there is no CPU fallback)")
         self.device = device
         self._corpora = weakref.WeakSet()  # sea_b200_corpus_destroy uses its context: they are closed before it
+        self._pools = weakref.WeakSet()  # so does sea_b200_encoder_pool_destroy
 
     def close(self):
         if getattr(self, "_h", None) and self._h.value:
             for corpus in list(getattr(self, "_corpora", ())):
                 corpus.close()
+            for pool in list(getattr(self, "_pools", ())):
+                pool.close()
             self._L.sea_b200_ctx_destroy(self._h)
             self._h = C.c_void_p()
 
@@ -437,6 +449,129 @@ class Context:
         """Registers the .sea streams held in `buf` (a uint8 CUDA tensor; streams described as for decode_windows_device) for
         Corpus.decode_windows.  Every chunk a window can cover is validated here, once."""
         return Corpus(self, buf, sea_offsets, sea_lens, headers, skip_metadata)
+
+    def encoder_pool(self, channels: int, sample_rate: int, settings: EncoderSettings, max_sessions: int) -> "EncoderPool":
+        """A slot table of max_sessions streaming encoders that share one launch per push (see EncoderPool)."""
+        return EncoderPool(self, channels, sample_rate, settings, max_sessions)
+
+
+class EncoderPool:
+    """Many live streams, one call per round of packets (sea_b200_encoder_pool): open(sessions) starts a stream in each slot, push()
+    appends a packet of any length to each listed session and returns every chunk that completed, and end=True also encodes the
+    rest as the session's short final chunk and frees the slot.  A session's .sea file is header(...) followed by its push outputs
+    joined, byte for byte what sea_encode gives for its whole PCM.  Keeps its Context alive; close() before the context's close."""
+
+    def __init__(self, ctx: Context, channels: int, sample_rate: int, settings: EncoderSettings, max_sessions: int):
+        self._h = C.c_void_p()
+        self._ctx, self._L = ctx, ctx._L
+        self.channels, self.sample_rate, self.settings, self.max_sessions = channels, sample_rate, settings, max_sessions
+        st = settings._c()
+        ctx._check(self._L.sea_b200_encoder_pool_create(ctx._h, max_sessions, channels, sample_rate, C.byref(st), C.byref(self._h)))
+        ctx._pools.add(self)
+        full = C.c_uint32(0)  # 0: a full chunk is outside the reference's domain at these settings (push reports it)
+        self._full = full.value if self._L.sea_b200_full_chunk_bytes(channels, C.byref(st), C.byref(full)) == OK else 0
+
+    def close(self):
+        if getattr(self, "_h", None) and self._h.value:
+            if self._ctx._h.value:  # as Corpus.close: never through a context the collector already destroyed
+                self._L.sea_b200_encoder_pool_destroy(self._h)
+            self._h = C.c_void_p()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    @staticmethod
+    def _sessions(sessions) -> np.ndarray:
+        return np.ascontiguousarray(np.atleast_1d(sessions), dtype=np.uint32)
+
+    @staticmethod
+    def _end(end, n: int):
+        if end is None:
+            return None
+        e = np.ascontiguousarray(np.broadcast_to(np.asarray(end, dtype=bool), (n,)), dtype=np.uint8)
+        return e
+
+    def open(self, sessions) -> None:
+        s = self._sessions(sessions)
+        self._ctx._check(self._L.sea_b200_encoder_pool_open(self._h, s.size, s.ctypes.data))
+
+    def buffered(self, sessions) -> np.ndarray:
+        """Frames each session holds back (fewer than frames_per_chunk; 0 for a closed slot)."""
+        s = self._sessions(sessions)
+        out = np.zeros(s.size, dtype=np.uint32)
+        self._ctx._check(self._L.sea_b200_encoder_pool_buffered(self._h, s.size, s.ctypes.data, out.ctypes.data))
+        return out
+
+    def push_bound(self, session: int, n_frames: int, end: bool = False) -> int:
+        b = C.c_uint64(0)
+        self._ctx._check(self._L.sea_b200_encoder_pool_push_bound(self._h, session, n_frames, bool(end), C.byref(b)))
+        return b.value
+
+    def header(self, session: int, first_chunk_bytes: int, total_frames: int) -> bytes:
+        """The 22-byte .sea header of a session's stream: chunk_size = the size of its first chunk (file.rs:166-168), total_frames
+        as the reference writes it (0 when the length was not known up front)."""
+        if not 0 <= session < self.max_sessions:
+            raise SeaError(ERR_INVALID_PARAMETERS, "session past max_sessions")
+        return _serialize_header(self.channels, first_chunk_bytes, self.settings.frames_per_chunk, self.sample_rate, total_frames)
+
+    def push(self, sessions, packets: Sequence[np.ndarray], end=None) -> List[bytes]:
+        """Appends packets[i] (interleaved int16) to session sessions[i]; returns per session the chunks that completed."""
+        s = self._sessions(sessions)
+        if len(packets) != s.size:
+            raise SeaError(ERR_INVALID_PARAMETERS, "one packet per session")
+        ch = self.channels
+        arrs = [np.ascontiguousarray(p, dtype=np.int16).reshape(-1) for p in packets]
+        if any(a.size % ch for a in arrs):
+            raise SeaError(ERR_INVALID_PARAMETERS, "packets must hold whole frames")
+        frames = np.array([a.size // ch for a in arrs], dtype=np.uint32)
+        pcm_off = np.zeros(s.size, dtype=np.uint64)
+        if s.size:
+            pcm_off[1:] = np.cumsum(frames.astype(np.uint64) * ch)[:-1]
+        pcm = np.concatenate(arrs) if arrs else np.zeros(0, np.int16)
+        pcm = pcm if pcm.size else np.zeros(1, np.int16)
+        e = self._end(end, s.size)
+        # chunks completed: exact; a final chunk: its bound
+        tot = self.buffered(s).astype(np.uint64) + frames
+        caps = tot // self.settings.frames_per_chunk * self._full
+        if e is not None:
+            for i in np.flatnonzero(e):
+                caps[i] = self.push_bound(int(s[i]), int(frames[i]), True)
+        out_off = np.zeros(s.size, dtype=np.uint64)
+        if s.size:
+            out_off[1:] = np.cumsum(caps)[:-1]
+        out = np.empty(int(caps.sum()) + 64, dtype=np.uint8)
+        lens = np.zeros(s.size, dtype=np.uint64)
+        self._ctx._check(self._L.sea_b200_encoder_pool_push(self._h, s.size, s.ctypes.data, pcm.ctypes.data, pcm_off.ctypes.data,
+                                                            frames.ctypes.data, e.ctypes.data if e is not None else None, out.ctypes.data,
+                                                            out_off.ctypes.data, caps.ctypes.data, lens.ctypes.data, None))
+        return [out[int(o): int(o) + int(n)].tobytes() for o, n in zip(out_off, lens)]
+
+    def push_host(self, sessions, pcm_ptr: int, pcm_offsets, n_frames, out_ptr: int, out_offsets, end=None, out_caps=None) -> np.ndarray:
+        """push() over caller-owned host buffers by raw address (pinned memory recommended); returns out_lens."""
+        return self._push(self._L.sea_b200_encoder_pool_push, sessions, pcm_ptr, pcm_offsets, n_frames, out_ptr, out_offsets, end, out_caps)
+
+    def push_device(self, sessions, d_pcm: int, pcm_offsets, n_frames, d_out: int, out_offsets, end=None, out_caps=None) -> np.ndarray:
+        """push() with the packets and the output in device memory (raw device pointers, e.g. tensor.data_ptr()); returns out_lens.
+        Bytes of d_out outside [out_offsets[i], + out_lens[i]) are never written."""
+        return self._push(self._L.sea_b200_encoder_pool_push_device, sessions, d_pcm, pcm_offsets, n_frames, d_out, out_offsets, end,
+                          out_caps)
+
+    def _push(self, fn, sessions, pcm_ptr, pcm_offsets, n_frames, out_ptr, out_offsets, end, out_caps) -> np.ndarray:
+        s = self._sessions(sessions)
+        po, oo = _u64(pcm_offsets), _u64(out_offsets)
+        nf = np.ascontiguousarray(n_frames, dtype=np.uint32)
+        if not (po.size == oo.size == nf.size == s.size):
+            raise SeaError(ERR_INVALID_PARAMETERS, "per-session arrays differ in length")
+        e = self._end(end, s.size)
+        caps = _u64(out_caps) if out_caps is not None else None
+        lens = np.zeros(s.size, dtype=np.uint64)
+        self._ctx._check(fn(self._h, s.size, s.ctypes.data, C.c_void_p(pcm_ptr), po.ctypes.data, nf.ctypes.data,
+                            e.ctypes.data if e is not None else None, C.c_void_p(out_ptr), oo.ctypes.data,
+                            caps.ctypes.data if caps is not None else None, lens.ctypes.data, None))
+        return lens
 
 
 class Corpus:

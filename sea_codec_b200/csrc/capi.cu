@@ -93,6 +93,27 @@ struct sea_b200_encoder {
     int32_t *d_state = nullptr;
 };
 
+// A slot table of streaming encoders that share one launch per push (sea_b200_encoder_pool_*).  Every slot owns a state row
+// (kEncStateWords int32 per channel) and two carry buffers of frames_per_chunk frames: a push that completes a chunk reads the
+// current carry into the launch input and writes the new remainder into the other one, so the ingest never reads what it writes.
+struct sea_b200_encoder_pool {
+    sea_b200_ctx *ctx;
+    sea_b200_settings settings;
+    EncodePlan plan;
+    uint32_t max_sessions, channels, sample_rate;
+    int16_t *d_carry = nullptr;  // [max_sessions][2][N * channels]
+    int32_t *d_state = nullptr;  // [max_sessions][channels * kEncStateWords]
+    int32_t *d_init = nullptr;   // one row of EncoderBase::new state: a freshly opened slot gathers its state from here
+    std::vector<uint32_t> carry;                 // frames buffered per slot
+    std::vector<uint8_t> half, open, fresh;      // current carry half; open; state row not yet written since open
+    std::vector<uint32_t> seen;                  // duplicate check: call stamp per slot
+    uint32_t stamp = 0;
+    DevBuf pk, in, rows, ob, desc;               // packets (host form), launch input, gathered state rows, output (host form), copies + slots
+    uint8_t *h_desc = nullptr;                   // pinned staging of the copy list and the slot list
+    size_t h_desc_cap = 0;
+    cudaEvent_t ev[4] = {};                      // ingest start, ingest end, encode end, commit end
+};
+
 struct sea_b200_decoder {
     sea_b200_ctx *ctx;
     sea_b200_header header;
@@ -1701,6 +1722,392 @@ int sea_b200_encoder_make_chunk(sea_b200_encoder *enc, const int16_t *pcm, uint6
     if (n_samples / (enc->channels ? enc->channels : 1) > enc->plan.N)
         return fail(enc->ctx, SEA_B200_ERR_DOMAIN, "more than frames_per_chunk frames (file.rs:173-175 assert)");
     return sea_b200_encoder_make_chunks(enc, pcm, n_samples, out, out_cap, out_len, nullptr);
+}
+
+// ------------------------------------------------------------------------------------------------ session pool
+
+int sea_b200_encoder_pool_create(sea_b200_ctx *ctx, uint32_t max_sessions, uint32_t channels, uint32_t sample_rate,
+                                 const sea_b200_settings *settings, sea_b200_encoder_pool **pool)
+{
+    if (!ctx || !settings || !pool) return SEA_B200_ERR_INVALID_PARAMETERS;
+    *pool = nullptr;
+    if (max_sessions == 0) return fail(ctx, SEA_B200_ERR_INVALID_PARAMETERS, "a pool needs at least one session slot");
+    EncodePlan pl;
+    int rc = make_encode_plan(channels, settings, &pl);
+    if (rc) return fail(ctx, rc, "encoder settings rejected (outside the reference's domain)");
+    CU(cudaSetDevice(ctx->device));
+    sea_b200_encoder_pool *p = new sea_b200_encoder_pool();
+    p->ctx = ctx;
+    p->settings = *settings;
+    p->plan = pl;
+    p->max_sessions = max_sessions;
+    p->channels = channels;
+    p->sample_rate = sample_rate;
+    auto bail = [&](cudaError_t e, const char *what) {
+        const int r = cuda_fail(ctx, e, what);
+        sea_b200_encoder_pool_destroy(p);
+        return r;
+    };
+    const size_t row = (size_t)channels * kEncStateWords;
+    cudaError_t e = cudaMalloc(&p->d_carry, (size_t)max_sessions * 2u * pl.N * channels * sizeof(int16_t));
+    if (e != cudaSuccess) return bail(e, "cudaMalloc(pool carry buffers)");
+    if ((e = cudaMalloc(&p->d_state, (size_t)max_sessions * row * sizeof(int32_t))) != cudaSuccess) return bail(e, "cudaMalloc(pool state)");
+    std::vector<int32_t> init(row, 0);
+    for (uint32_t c = 0; c < channels; c++) {  // lms.rs:19-32
+        init[(size_t)c * kEncStateWords + 4 + 2] = -(1 << 13);
+        init[(size_t)c * kEncStateWords + 4 + 3] = 1 << 14;
+    }
+    if ((e = cudaMalloc(&p->d_init, row * sizeof(int32_t))) != cudaSuccess) return bail(e, "cudaMalloc(pool initial state)");
+    if ((e = cudaMemcpy(p->d_init, init.data(), row * sizeof(int32_t), cudaMemcpyHostToDevice)) != cudaSuccess)
+        return bail(e, "cudaMemcpy(pool initial state)");
+    for (cudaEvent_t &ev : p->ev)
+        if ((e = cudaEventCreate(&ev)) != cudaSuccess) return bail(e, "cudaEventCreate");
+    p->carry.assign(max_sessions, 0);
+    p->half.assign(max_sessions, 0);
+    p->open.assign(max_sessions, 0);
+    p->fresh.assign(max_sessions, 1);
+    p->seen.assign(max_sessions, 0);
+    *pool = p;
+    return SEA_B200_OK;
+}
+
+void sea_b200_encoder_pool_destroy(sea_b200_encoder_pool *pool)
+{
+    if (!pool) return;
+    cudaSetDevice(pool->ctx->device);
+    if (pool->ctx->stream) cudaStreamSynchronize(pool->ctx->stream);
+    if (pool->d_carry) cudaFree(pool->d_carry);
+    if (pool->d_state) cudaFree(pool->d_state);
+    if (pool->d_init) cudaFree(pool->d_init);
+    pool->pk.release();
+    pool->in.release();
+    pool->rows.release();
+    pool->ob.release();
+    pool->desc.release();
+    if (pool->h_desc) cudaFreeHost(pool->h_desc);
+    for (cudaEvent_t ev : pool->ev)
+        if (ev) cudaEventDestroy(ev);
+    delete pool;
+}
+
+int sea_b200_encoder_pool_open(sea_b200_encoder_pool *pool, uint32_t n, const uint32_t *sessions)
+{
+    if (!pool) return SEA_B200_ERR_INVALID_PARAMETERS;
+    sea_b200_ctx *ctx = pool->ctx;
+    if (n == 0) return SEA_B200_OK;
+    if (!sessions) return fail(ctx, SEA_B200_ERR_INVALID_PARAMETERS, "NULL session list");
+    if (++pool->stamp == 0) {
+        std::fill(pool->seen.begin(), pool->seen.end(), 0u);
+        pool->stamp = 1;
+    }
+    for (uint32_t i = 0; i < n; i++) {
+        const uint32_t s = sessions[i];
+        if (s >= pool->max_sessions || pool->open[s] || pool->seen[s] == pool->stamp)
+            return fail(ctx, SEA_B200_ERR_INVALID_PARAMETERS, "session " + std::to_string(s) + " (entry " + std::to_string(i) + ")" +
+                                                                  (s >= pool->max_sessions ? " is past max_sessions" : pool->open[s] ? " is already open" : " appears twice"));
+        pool->seen[s] = pool->stamp;
+    }
+    // host-side only: the slot's first push gathers its state from the EncoderBase::new row
+    for (uint32_t i = 0; i < n; i++) {
+        const uint32_t s = sessions[i];
+        pool->open[s] = 1;
+        pool->fresh[s] = 1;
+        pool->carry[s] = 0;
+        pool->half[s] = 0;
+    }
+    return SEA_B200_OK;
+}
+
+int sea_b200_encoder_pool_buffered(const sea_b200_encoder_pool *pool, uint32_t n, const uint32_t *sessions, uint32_t *frames)
+{
+    if (!pool) return SEA_B200_ERR_INVALID_PARAMETERS;
+    if (n && (!sessions || !frames)) return fail(pool->ctx, SEA_B200_ERR_INVALID_PARAMETERS, "NULL pointer");
+    for (uint32_t i = 0; i < n; i++)
+        if (sessions[i] >= pool->max_sessions) return fail(pool->ctx, SEA_B200_ERR_INVALID_PARAMETERS, "session past max_sessions");
+    for (uint32_t i = 0; i < n; i++) frames[i] = pool->open[sessions[i]] ? pool->carry[sessions[i]] : 0u;
+    return SEA_B200_OK;
+}
+
+}  // extern "C"
+
+namespace {
+
+// Bytes a push of n_frames more frames gives an open session: k full chunks, plus with `end` the bound of its short final chunk
+// (exact for CBR; sea_b200_encode_bound's for VBR, whose last chunk size is only known once it is encoded).
+uint64_t pool_bound(const EncodePlan &pl, uint64_t total_frames, bool end)
+{
+    if (end) return encode_bound_bytes(pl, total_frames) - kFileHeaderBytes;
+    return total_frames / pl.N * pl.full_chunk_bytes;
+}
+
+int pool_push(sea_b200_encoder_pool *pool, uint32_t n, const uint32_t *sessions, const int16_t *pcm, const uint64_t *pcm_offsets,
+              const uint32_t *n_frames, const uint8_t *end, uint8_t *out, const uint64_t *out_offsets, const uint64_t *out_caps,
+              uint64_t *out_lens, uint32_t *n_chunks, bool device)
+{
+    if (!pool) return SEA_B200_ERR_INVALID_PARAMETERS;
+    sea_b200_ctx *ctx = pool->ctx;
+    if (n == 0) return SEA_B200_OK;
+    if (!sessions || !pcm_offsets || !n_frames || !out_offsets || !out_lens) return fail(ctx, SEA_B200_ERR_INVALID_PARAMETERS, "NULL pointer");
+    const EncodePlan &pl = pool->plan;
+    const uint32_t C = pool->channels, N = pl.N, row = C * kEncStateWords;
+    const uint64_t slot_elems = (uint64_t)N * C;
+
+    // ---- every refusal comes before anything is enqueued or any session's bookkeeping moves
+    if (++pool->stamp == 0) {
+        std::fill(pool->seen.begin(), pool->seen.end(), 0u);
+        pool->stamp = 1;
+    }
+    std::vector<uint32_t> enc_frames(n);
+    std::vector<uint64_t> bound(n);
+    uint64_t lo = UINT64_MAX, hi = 0, out_total = 0;
+    bool vbr_tail = false;  // some session ends with a VBR short chunk: its size is read back before the output can be copied
+    for (uint32_t i = 0; i < n; i++) {
+        const uint32_t s = sessions[i];
+        auto who = [&]() { return "session " + std::to_string(s) + " (entry " + std::to_string(i) + ")"; };
+        if (s >= pool->max_sessions) return fail(ctx, SEA_B200_ERR_INVALID_PARAMETERS, who() + " is past max_sessions");
+        if (!pool->open[s]) return fail(ctx, SEA_B200_ERR_INVALID_PARAMETERS, who() + " is not open");
+        if (pool->seen[s] == pool->stamp) return fail(ctx, SEA_B200_ERR_INVALID_PARAMETERS, who() + " appears twice in one push");
+        pool->seen[s] = pool->stamp;
+        const uint64_t tot = (uint64_t)pool->carry[s] + n_frames[i];
+        if (tot > 0xffffffffull) return fail(ctx, SEA_B200_ERR_TOO_MANY_FRAMES, who() + ": buffered plus pushed frames exceed 2^32");
+        const bool e = end && end[i];
+        enc_frames[i] = (uint32_t)(e ? tot : tot / N * N);
+        bound[i] = pool_bound(pl, tot, e);
+        if (out_caps && out_caps[i] < bound[i])
+            return fail(ctx, SEA_B200_ERR_CAPACITY, who() + ": out_caps smaller than sea_b200_encoder_pool_push_bound");
+        if (e && pl.vbr && tot % N) vbr_tail = true;
+        if (n_frames[i]) {
+            lo = std::min(lo, pcm_offsets[i]);
+            hi = std::max(hi, pcm_offsets[i] + (uint64_t)n_frames[i] * C);
+        }
+        out_total += bound[i];
+    }
+    if (hi && !pcm) return fail(ctx, SEA_B200_ERR_INVALID_PARAMETERS, "NULL pcm");
+    if (out_total && !out) return fail(ctx, SEA_B200_ERR_INVALID_PARAMETERS, "NULL out");
+    if (hi == 0) lo = 0;
+
+    // ---- the encode launch: one stream per session that completes a chunk or ends with frames, in call order
+    std::vector<uint32_t> launch;  // call index of launch stream j
+    std::vector<uint64_t> in_off, enc_out_off;
+    std::vector<uint32_t> frames_j;
+    uint64_t in_total = 0, ob_total = 0;
+    for (uint32_t i = 0; i < n; i++) {
+        if (!enc_frames[i]) continue;
+        launch.push_back(i);
+        in_off.push_back(in_total);
+        in_total += ((uint64_t)enc_frames[i] * C + 7u) & ~7ull;  // 16-byte aligned rows: whole-vector stores for most of them
+        frames_j.push_back(enc_frames[i]);
+        enc_out_off.push_back(device ? out_offsets[i] : ob_total);
+        ob_total += bound[i];
+    }
+    const uint32_t nl = (uint32_t)launch.size();
+    EncodeJob job;
+    if (nl) {
+        int rc = plan_encode(ctx, nl, in_off.data(), frames_j.data(), pool->sample_rate, C, &pool->settings, enc_out_off.data(), true, &job);
+        if (rc) return rc;
+    }
+    CU(cudaSetDevice(ctx->device));
+    // pinned staging: the copy list (at most three copies and a state row per session), the launch's slots, its EncStreams
+    const size_t max_copies = (size_t)n * 3u + nl;
+    const size_t enc_at = (sizeof(PoolCopy) * max_copies + sizeof(uint32_t) * nl + 15u) & ~(size_t)15u;
+    const size_t desc_bytes = enc_at + sizeof(EncStream) * nl;
+    CU(pool->desc.reserve(desc_bytes));
+    if (pool->h_desc_cap < desc_bytes) {
+        if (pool->h_desc) cudaFreeHost(pool->h_desc);
+        pool->h_desc = nullptr;
+        pool->h_desc_cap = 0;
+        CU(cudaHostAlloc(reinterpret_cast<void **>(&pool->h_desc), desc_bytes + (desc_bytes >> 2), cudaHostAllocDefault));
+        pool->h_desc_cap = desc_bytes + (desc_bytes >> 2);
+    }
+    CU(pool->in.reserve(in_total * sizeof(int16_t) + 64));
+    CU(pool->rows.reserve((size_t)nl * row * sizeof(int32_t) + 64));
+    if (!device) {
+        CU(pool->pk.reserve((hi - lo) * sizeof(int16_t) + 64));
+        CU(pool->ob.reserve(ob_total + 64));
+    }
+    if (nl) {
+        CU(ctx->streams.reserve(sizeof(EncStream) * nl));
+        CU(ctx->lens.reserve(sizeof(uint64_t) * nl));
+        CU(ctx->chunk0.reserve(sizeof(uint32_t) * nl));
+        CU(ctx->ties.reserve(sizeof(unsigned long long) * ((size_t)nl + 1u)));
+    }
+
+    // ---- the ingest's copies, in call order (device pointers are final now)
+    PoolCopy *copies = reinterpret_cast<PoolCopy *>(pool->h_desc);
+    uint32_t n_copies = 0;
+    uint64_t vectors = 0;
+    auto add = [&](const int16_t *src, int16_t *dst, uint64_t elems) {
+        if (!elems) return;
+        PoolCopy &c = copies[n_copies++];
+        c.src = src;
+        c.dst = dst;
+        c.n = elems;
+        c.v_begin = vectors;
+        const uint64_t d = reinterpret_cast<uintptr_t>(dst);
+        vectors += ((d + 2u * elems + 15u) >> 4) - (d >> 4);
+    };
+    int16_t *d_in = pool->in.as<int16_t>();
+    int32_t *d_rows = pool->rows.as<int32_t>();
+    for (uint32_t i = 0, j = 0; i < n; i++) {
+        const uint32_t s = sessions[i], c = pool->carry[s];
+        const int16_t *packet = !n_frames[i] ? nullptr : device ? pcm + pcm_offsets[i] : pool->pk.as<int16_t>() + (pcm_offsets[i] - lo);
+        int16_t *cur = pool->d_carry + ((uint64_t)s * 2u + pool->half[s]) * slot_elems;
+        int16_t *nxt = pool->d_carry + ((uint64_t)s * 2u + (pool->half[s] ^ 1u)) * slot_elems;
+        if (!enc_frames[i]) {  // no chunk completes: the packet is appended behind the carry, in place
+            add(packet, cur + (uint64_t)c * C, (uint64_t)n_frames[i] * C);
+            continue;
+        }
+        // carry + the packet's first enc_frames - c frames -> launch input; the remainder -> the other carry half
+        int16_t *dst = d_in + in_off[j];
+        const uint64_t take = enc_frames[i] - c, rest = (uint64_t)c + n_frames[i] - enc_frames[i];
+        add(cur, dst, (uint64_t)c * C);
+        add(packet, dst + (uint64_t)c * C, take * C);
+        if (rest) add(packet + take * C, nxt, rest * C);
+        const int32_t *src_row = pool->fresh[s] ? pool->d_init : pool->d_state + (uint64_t)s * row;
+        add(reinterpret_cast<const int16_t *>(src_row), reinterpret_cast<int16_t *>(d_rows + (uint64_t)j * row), 2ull * row);
+        j++;
+    }
+    uint32_t *slots = reinterpret_cast<uint32_t *>(pool->h_desc + sizeof(PoolCopy) * n_copies);
+    for (uint32_t j = 0; j < nl; j++) slots[j] = sessions[launch[j]];
+    if (nl) memcpy(pool->h_desc + enc_at, job.streams.data(), sizeof(EncStream) * nl);
+    const PoolCopy *d_copies = pool->desc.as<PoolCopy>();
+    const uint32_t *d_slots = reinterpret_cast<const uint32_t *>(pool->desc.as<uint8_t>() + sizeof(PoolCopy) * n_copies);
+
+    // ---- enqueue, wait, copy back.  From here on a failure leaves the device state of the call's sessions undefined: they are
+    // closed.
+    std::vector<unsigned long long> dev_ties;
+    std::vector<uint64_t> lens_j(nl);
+    auto run = [&]() -> int {
+        cudaStream_t st = ctx->stream;
+        if (!device && hi) CU(cudaMemcpyAsync(pool->pk.p, pcm + lo, (hi - lo) * sizeof(int16_t), cudaMemcpyHostToDevice, st));
+        CU(cudaMemcpyAsync(pool->desc.p, pool->h_desc, sizeof(PoolCopy) * n_copies + sizeof(uint32_t) * nl, cudaMemcpyHostToDevice, st));
+        if (nl) CU(cudaMemcpyAsync(ctx->streams.p, pool->h_desc + enc_at, sizeof(EncStream) * nl, cudaMemcpyHostToDevice, st));
+        CU(cudaEventRecord(pool->ev[0], st));
+        if (n_copies) {
+            CU(launch_pool_ingest(d_copies, n_copies, vectors, st));
+            ctx->launches++;
+        }
+        CU(cudaEventRecord(pool->ev[1], st));
+        int dev_err = 0;
+        if (nl) {
+            CU(cudaMemsetAsync(ctx->d_err, 0, sizeof(int), st));
+            CU(cudaMemsetAsync(ctx->ties.p, 0, sizeof(unsigned long long) * ((size_t)nl + 1u), st));
+            int rc = enqueue_encode(ctx, job, d_in, device ? out : pool->ob.as<uint8_t>(), d_rows, 0, true);
+            if (rc) return rc;
+            CU(cudaEventRecord(pool->ev[2], st));
+            CU(launch_pool_commit(d_rows, pool->d_state, d_slots, nl, row, st));
+            ctx->launches++;
+            CU(cudaEventRecord(pool->ev[3], st));
+            CU(cudaMemcpyAsync(&dev_err, ctx->d_err, sizeof(int), cudaMemcpyDeviceToHost, st));
+            if (pl.vbr) {
+                dev_ties.assign((size_t)nl + 1u, 0ull);
+                CU(cudaMemcpyAsync(dev_ties.data(), ctx->ties.p, sizeof(unsigned long long) * ((size_t)nl + 1u), cudaMemcpyDeviceToHost, st));
+            }
+            if (vbr_tail) CU(cudaMemcpyAsync(lens_j.data(), ctx->lens.p, sizeof(uint64_t) * nl, cudaMemcpyDeviceToHost, st));
+        } else {
+            CU(cudaEventRecord(pool->ev[2], st));
+            CU(cudaEventRecord(pool->ev[3], st));
+        }
+        // a full chunk is full_chunk_bytes exactly and a CBR short chunk follows from its frame count: those sizes are known here,
+        // and the output goes back in the same stream segment; a VBR short chunk has to be read back first
+        auto copy_back = [&]() -> int {
+            if (device) return SEA_B200_OK;
+            for (uint32_t j = 0; j < nl;) {  // one copy per run of sessions adjacent both in the staging buffer and in `out`
+                uint32_t k = j + 1;
+                uint64_t len = lens_j[j];
+                while (k < nl && enc_out_off[k] == enc_out_off[j] + len && out_offsets[launch[k]] == out_offsets[launch[j]] + len) len += lens_j[k++];
+                if (len) CU(cudaMemcpyAsync(out + out_offsets[launch[j]], pool->ob.as<uint8_t>() + enc_out_off[j], len, cudaMemcpyDeviceToHost, st));
+                j = k;
+            }
+            return SEA_B200_OK;
+        };
+        if (!vbr_tail) {
+            for (uint32_t j = 0; j < nl; j++) {
+                const uint32_t f = frames_j[j], rem = f % N;
+                lens_j[j] = (uint64_t)(f / N) * pl.full_chunk_bytes + (rem ? cbr_chunk_bytes(rem, C, pl.s, pl.F, pl.hdr_bits) : 0u);
+            }
+            if (int rc = copy_back()) return rc;
+        }
+        CU(cudaStreamSynchronize(st));
+        if (dev_err != kDevOk) return map_dev_error(ctx, dev_err);
+        if (vbr_tail) {
+            if (int rc = copy_back()) return rc;
+            CU(cudaStreamSynchronize(st));
+        }
+        return SEA_B200_OK;
+    };
+    const int rc = run();
+    if (rc != SEA_B200_OK) {
+        for (uint32_t i = 0; i < n; i++) {
+            pool->open[sessions[i]] = 0;
+            pool->carry[sessions[i]] = 0;
+        }
+        return rc;
+    }
+
+    // ---- results and the sessions' bookkeeping
+    float ms[3] = {0.f, 0.f, 0.f};
+    cudaEventElapsedTime(&ms[0], pool->ev[0], pool->ev[1]);
+    cudaEventElapsedTime(&ms[1], pool->ev[1], pool->ev[2]);
+    cudaEventElapsedTime(&ms[2], pool->ev[2], pool->ev[3]);
+    ctx->last_kernel_ms = (double)ms[0] + ms[1] + ms[2];
+    if (getenv("SEA_B200_TRACE"))
+        fprintf(stderr, "sea_b200 trace: pool push: %u sessions, %u encode, %u copies; ingest %.3f ms, encode %.3f ms, commit %.3f ms\n", n, nl,
+                n_copies, ms[0], ms[1], ms[2]);
+    ctx->h_ties.assign((size_t)n + 1u, 0ull);  // call order
+    for (uint32_t j = 0; j < nl && pl.vbr; j++) ctx->h_ties[1u + launch[j]] = dev_ties[1u + j];
+    ctx->h_ties[0] = pl.vbr && nl ? dev_ties[0] : 0ull;
+    ctx->last_ties = ctx->h_ties[0];
+    for (uint32_t i = 0; i < n; i++) {
+        out_lens[i] = 0;
+        if (n_chunks) n_chunks[i] = (enc_frames[i] + N - 1u) / N;
+    }
+    for (uint32_t j = 0; j < nl; j++) out_lens[launch[j]] = lens_j[j];
+    for (uint32_t i = 0; i < n; i++) {
+        const uint32_t s = sessions[i];
+        const uint64_t tot = (uint64_t)pool->carry[s] + n_frames[i];
+        if (end && end[i]) {
+            pool->open[s] = 0;
+            pool->carry[s] = 0;
+        } else if (enc_frames[i]) {
+            pool->carry[s] = (uint32_t)(tot - enc_frames[i]);
+            pool->half[s] ^= 1u;
+        } else {
+            pool->carry[s] = (uint32_t)tot;
+        }
+        if (enc_frames[i]) pool->fresh[s] = 0;
+    }
+    return SEA_B200_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int sea_b200_encoder_pool_push_bound(const sea_b200_encoder_pool *pool, uint32_t session, uint64_t n_frames, bool end, uint64_t *bytes)
+{
+    if (!pool || !bytes) return SEA_B200_ERR_INVALID_PARAMETERS;
+    if (session >= pool->max_sessions || !pool->open[session])
+        return fail(pool->ctx, SEA_B200_ERR_INVALID_PARAMETERS, "session " + std::to_string(session) + " is not open");
+    const uint64_t tot = pool->carry[session] + n_frames;
+    if (n_frames > 0xffffffffull || tot > 0xffffffffull)
+        return fail(pool->ctx, SEA_B200_ERR_TOO_MANY_FRAMES, "buffered plus pushed frames exceed 2^32");
+    *bytes = pool_bound(pool->plan, tot, end);
+    return SEA_B200_OK;
+}
+
+int sea_b200_encoder_pool_push(sea_b200_encoder_pool *pool, uint32_t n, const uint32_t *sessions, const int16_t *pcm,
+                               const uint64_t *pcm_offsets, const uint32_t *n_frames, const uint8_t *end, uint8_t *out,
+                               const uint64_t *out_offsets, const uint64_t *out_caps, uint64_t *out_lens, uint32_t *n_chunks)
+{
+    return pool_push(pool, n, sessions, pcm, pcm_offsets, n_frames, end, out, out_offsets, out_caps, out_lens, n_chunks, false);
+}
+
+int sea_b200_encoder_pool_push_device(sea_b200_encoder_pool *pool, uint32_t n, const uint32_t *sessions, const int16_t *d_pcm,
+                                      const uint64_t *pcm_offsets, const uint32_t *n_frames, const uint8_t *end, uint8_t *d_out,
+                                      const uint64_t *out_offsets, const uint64_t *out_caps, uint64_t *out_lens, uint32_t *n_chunks)
+{
+    return pool_push(pool, n, sessions, d_pcm, pcm_offsets, n_frames, end, d_out, out_offsets, out_caps, out_lens, n_chunks, true);
 }
 
 int sea_b200_decoder_create(sea_b200_ctx *ctx, const uint8_t *header22, uint64_t len, sea_b200_decoder **out)

@@ -198,6 +198,20 @@ cudaError_t launch_encode_generic(const int16_t *d_pcm, uint8_t *d_out, const En
                                   DevTables tabs, int32_t *d_state, uint64_t *d_out_lens, uint32_t *d_chunk0,
                                   unsigned long long *d_ties, EncWorkspace ws, int *d_err, cudaStream_t stream, uint32_t chunk_buf_bytes);
 
+// ---- session pool (pool_kernels.cu, sea_b200_encoder_pool_push) ---------------------------------------------
+// One copy of the ingest: n int16 elements (n > 0) from src to dst, both in device memory, 2-byte aligned, not overlapping any
+// other copy of the launch.  v_begin: the number of 16-byte destination vectors the copies before this one touch.
+struct PoolCopy {
+    const int16_t *src;
+    int16_t *dst;
+    uint64_t n;
+    uint64_t v_begin;
+};
+cudaError_t launch_pool_ingest(const PoolCopy *d_copies, uint32_t n_copies, uint64_t total_vectors, cudaStream_t stream);
+// rows: n_rows state rows of row_words int32 in launch order; row r goes to state + slots[r] * row_words.
+cudaError_t launch_pool_commit(const int32_t *d_rows, int32_t *d_state, const uint32_t *d_slots, uint32_t n_rows, uint32_t row_words,
+                               cudaStream_t stream);
+
 // ---- measurement -------------------------------------------------------------------------------------------
 cudaError_t launch_int32_peak(int mode, uint32_t *d_sink, uint64_t *lane_ops, cudaStream_t stream);
 // synthetic tone + noise PCM of sea_codec_b200/synth.py, generated in place on the device (bench inputs)
